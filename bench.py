@@ -29,6 +29,24 @@ sys.path.insert(0, ROOT)
 
 METRIC = "fwd+inv dynamics evals/s (Tello, batch 2^20)"
 UNIT = "fwd+inv state evaluations/s"
+# --dump-outputs writes at most this many bytes: beyond it, a fixed seeded sample of the states (rows)
+DUMP_BYTES = 48 << 20
+
+
+def dump_rows(n, cols):
+    """Sorted indices of the rows of [n, cols] float64 outputs that --dump-outputs writes: every row if they fit
+    DUMP_BYTES, otherwise the same seeded sample on every run."""
+    k = DUMP_BYTES // (8 * cols)
+    if n <= k:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(0).choice(n, k, replace=False))
+
+
+def dump_outputs(out_dir, arrays):
+    """arrays: name -> float64 array (the sampled rows of one output), written as out_dir/<name>.npy."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, dtype=np.float64))
 
 
 def load_peaks():
@@ -108,8 +126,11 @@ def run_reference(args):
     t0 = time.perf_counter()
     for _ in range(args.steps):
         ydd = o.forward_dynamics(q, yd, tau, threads=cores)
-        o.inverse_dynamics(q, yd, ydd, threads=cores)
+        tau_back = o.inverse_dynamics(q, yd, ydd, threads=cores)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        rows = dump_rows(n, 2 * o.nv)
+        dump_outputs(args.dump_outputs, {"ydd": ydd[rows], "tau_back": tau_back[rows]})
     value = n * args.steps / dt
     line = {"impl": "reference", "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": args.gpus,
             "steps": args.steps, "warmup": args.warmup, "ms_per_step": 1e3 * dt / args.steps,
@@ -173,7 +194,13 @@ def main():
     ap.add_argument("--scaling", choices=("weak", "strong"), default="weak",
                     help="weak: --batch states per GPU; strong: --batch states in total, sharded")
     ap.add_argument("--no-extras", action="store_true", help="skip the config-3 leg and the depth sweep")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step (ydd of forwardDynamics, tau_back of inverseDynamics; "
+                         "rank 0's shard, a fixed seeded sample of its states beyond %d MB) as DIR/<name>.npy, float64"
+                         % (DUMP_BYTES >> 20))
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
 
     if args.impl == "reference":
@@ -253,6 +280,12 @@ def main():
     barrier()
     launches = grbda.launch_count() - launches0
     ms = e0.elapsed_time(e1)
+    dumped = None
+    if args.dump_outputs and rank == 0:
+        # copied before anything else runs: these are the buffers the last timed step wrote
+        rows = torch.from_numpy(dump_rows(B if primary is step else Bs, 2 * m.nv)).to(dev)
+        dumped = {"ydd": ydd.index_select(0, rows).cpu().numpy(),
+                  "tau_back": tau_back.index_select(0, rows).cpu().numpy()}
     # The timed region lasts ~20 ms, one nvidia-smi query takes longer than that: the sampler keeps running
     # over an untimed continuation of exactly the same steps (about 0.7 s) so that the clocks / throttle
     # reasons reported are a median over several samples under this load.
@@ -445,6 +478,8 @@ def main():
                                    "bytes_per_state": 8 * (m.nq + m.nv + 18 * m.nb),
                                    "hbm_frac": 8 * (m.nq + m.nv + 18 * m.nb) * Bk / t_fk / 1e9 / peaks["hbm_gbs"]}}
         line["other_kernels"].update(extras)
+        if dumped:
+            dump_outputs(args.dump_outputs, dumped)
         emit(line)
     if world > 1:
         dist.barrier()

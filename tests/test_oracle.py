@@ -31,20 +31,6 @@ def test_oracle_matches_reference_generated_dynamics(oracle, case, suffix):
         assert rel(m.inverse_dynamics(y, yd, ydd_ref, threads=1), tau_ref) < 1e-11
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference"), reason="reference sources only exist in the build container")
-def test_oracle_matches_live_reference_codegen(oracle):
-    """Same check against the freshly compiled oracle/_ref library on new random states."""
-    oracle.build()
-    rng = np.random.default_rng(5)
-    for case in KAT["cases"]:
-        m = oracle.OracleModel(case["robot"])
-        n = case["n"]
-        for _ in range(50):
-            y, yd, tau = (rng.uniform(-1, 1, (1, n)) for _ in range(3))
-            ref = oracle.reference_codegen(case["function_prefix"] + "FwdDyn", [y[0], yd[0], tau[0]], n)
-            assert rel(m.forward_dynamics(y, yd, tau, threads=1)[0], ref) < 1e-11
-
-
 def test_appendix_d_vectors(oracle):
     """SURVEY Appendix D: values obtained by running the reference's generated C."""
     m = oracle.OracleModel("revolute_chain_with_rotor_2")
