@@ -32,6 +32,7 @@ ALGO_NAMES = ["id", "fd", "fk", "h", "phi"]
 ALGO_GFA, ALGO_GFS = 5, 6  # tau_in +/- J^T f_ext (external forces on the terminal links)
 ALGO_CONTACT_KIN, ALGO_CONTACT_JAC, ALGO_TEST_FORCE, ALGO_OSIM = 8, 9, 10, 11  # operational space (contact points)
 ALGO_ID_DERIV, ALGO_FD_DERIV = 12, 13  # derivatives of the dynamics
+ALGO_ID_VJP, ALGO_FD_VJP = 14, 15  # vector-Jacobian products of the dynamics (reverse mode)
 PROGRAM_FD_LTL = 7  # dump_program only: forward dynamics as CRBA + bias + sparse L^T D L (kernel variant "ltl")
 
 _vp = C.c_void_p
@@ -78,6 +79,8 @@ _lib.grbda_cuda_apply_test_force_f64.argtypes = [_vp, _vp, _vp, _vp, _vp, _i64, 
 _lib.grbda_cuda_inverse_osim_f64.argtypes = [_vp, _vp, _vp, _i64, _vp]
 _lib.grbda_cuda_inverse_dynamics_derivatives_f64.argtypes = [_vp, _vp, _vp, _vp, _vp, _vp, _i64, _vp]
 _lib.grbda_cuda_forward_dynamics_derivatives_f64.argtypes = [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _vp]
+_lib.grbda_cuda_inverse_dynamics_vjp_f64.argtypes = [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _vp]
+_lib.grbda_cuda_forward_dynamics_vjp_f64.argtypes = [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _vp]
 _lib.grbda_cuda_integrate_f64.argtypes = [_vp, _vp, _vp, _vp, C.c_double, _vp, _vp, _vp, _i64, _vp]
 _lib.grbda_cuda_step_f64.argtypes = [_vp, _vp, _vp, _vp, _vp, C.c_double, _vp, _vp, _vp, _i64, _vp]
 _lib.grbda_cuda_dynamics_host_f64.argtypes = [_vp, C.c_int, _vp, _vp, _vp, _vp, _i64]
@@ -101,6 +104,7 @@ EXPORTED_SYMBOLS = [
     "grbda_cuda_contact_kinematics_f64", "grbda_cuda_contact_jacobians_f64", "grbda_cuda_apply_test_force_f64",
     "grbda_cuda_inverse_osim_f64",
     "grbda_cuda_inverse_dynamics_derivatives_f64", "grbda_cuda_forward_dynamics_derivatives_f64",
+    "grbda_cuda_inverse_dynamics_vjp_f64", "grbda_cuda_forward_dynamics_vjp_f64",
     "grbda_cuda_inverse_dynamics_f64", "grbda_cuda_inverse_dynamics_f32",
     "grbda_cuda_forward_dynamics_f64", "grbda_cuda_forward_dynamics_f32",
     "grbda_cuda_mass_matrix_f64", "grbda_cuda_mass_matrix_f32",
@@ -568,6 +572,26 @@ class ClusterTreeModel:
                                                                 _ptr(dt), q.shape[0], _stream()))
         return dq.transpose(1, 2), dv.transpose(1, 2), dt.transpose(1, 2)
 
+    def _vjp(self, name, q, yd, aux, w):
+        import torch
+        q = self._prep(q, self.nq, torch.float64)
+        yd, aux, w = (self._prep(t, self.nv, torch.float64) for t in (yd, aux, w))
+        q_bar = torch.empty_like(q)
+        yd_bar, aux_bar = torch.empty_like(yd), torch.empty_like(yd)
+        _check(getattr(_lib, name)(self._h, _ptr(q), _ptr(yd), _ptr(aux), _ptr(w), _ptr(q_bar), _ptr(yd_bar),
+                                   _ptr(aux_bar), q.shape[0], _stream()))
+        return q_bar, yd_bar, aux_bar
+
+    def inverseDynamicsVJP(self, q, yd, ydd, tau_bar):
+        """(q_bar[batch, nq], yd_bar[batch, nv], ydd_bar[batch, nv]): the cotangent tau_bar of tau = ID(q, yd, ydd)
+        pulled back to the inputs (ydd_bar = H tau_bar); q_bar is the gradient with respect to the stored positions."""
+        return self._vjp("grbda_cuda_inverse_dynamics_vjp_f64", q, yd, ydd, tau_bar)
+
+    def forwardDynamicsVJP(self, q, yd, tau, ydd_bar):
+        """(q_bar[batch, nq], yd_bar[batch, nv], tau_bar[batch, nv]): the cotangent ydd_bar of ydd = FD(q, yd, tau)
+        pulled back to the inputs (tau_bar = H^-1 ydd_bar); q_bar as documented in include/grbda_cuda.h."""
+        return self._vjp("grbda_cuda_forward_dynamics_vjp_f64", q, yd, tau, ydd_bar)
+
     def integrate(self, q, yd, ydd, dt, out=None):
         """(q', yd', flags): semi-implicit Euler step, quaternion base by ori::integrateQuat, implicit clusters
         projected back onto phi = 0; flags[b] = 1 where that projection failed."""
@@ -691,3 +715,11 @@ def checksum(x):
     x = x.contiguous()
     _check(_lib.grbda_cuda_checksum_f64(_ptr(x), x.numel(), out, _stream()))
     return out[0], out[1]
+
+
+def __getattr__(name):
+    # grbda.autograd imports torch: loaded on first use, so that importing the package does not
+    if name == "autograd":
+        import importlib
+        return importlib.import_module(__name__ + ".autograd")
+    raise AttributeError("module %r has no attribute %r" % (__name__, name))

@@ -869,6 +869,80 @@ namespace grbda
             }
 
             // ---------------------------------------------------------------------------------
+            // reverse mode: vector-Jacobian products of the dynamics. The cotangent w travels in input array 2
+            // behind the third argument, [aux (nv); w (nv)]. q_bar is the gradient with respect to the STORED
+            // position entries (nq of them, what torch.autograd needs): q_bar[k] = sum_i w_i d out_i / d q[k].
+            // ---------------------------------------------------------------------------------
+            std::vector<Sym> vjpPositions() const
+            {
+                std::vector<Sym> x(m_.getNumPositions());
+                for (int k = 0; k < (int)x.size(); k++)
+                    x[k] = Sym::input(IN_Q, k);
+                return x;
+            }
+            std::vector<Sym> vjpCotangent() const
+            {
+                const int nv = m_.getNumDegreesOfFreedom();
+                std::vector<Sym> w(nv);
+                for (int i = 0; i < nv; i++)
+                    w[i] = Sym::input(IN_AUX, nv + i);
+                return w;
+            }
+
+            // in2 = [ydd; tau_bar]: (q_bar, yd_bar, ydd_bar = H tau_bar), one reverse sweep of the inverse dynamics.
+            // q_bar is the exact derivative of the inverse-dynamics program for every position entry, also off the
+            // unit quaternion and off phi = 0.
+            void inverseDynamicsVJP(std::vector<Sym> &q_bar, std::vector<Sym> &yd_bar, std::vector<Sym> &ydd_bar)
+            {
+                const int nq = m_.getNumPositions(), nv = m_.getNumDegreesOfFreedom();
+                const std::vector<Sym> tau = inverseDynamics();
+                std::vector<Sym> wrt = vjpPositions();
+                for (int i = 0; i < nv; i++)
+                    wrt.push_back(inYd(i));
+                for (int i = 0; i < nv; i++)
+                    wrt.push_back(inAux(i));
+                const std::vector<Sym> bar = adjointSweep(tau, vjpCotangent(), wrt);
+                q_bar.assign(bar.begin(), bar.begin() + nq);
+                yd_bar.assign(bar.begin() + nq, bar.begin() + nq + nv);
+                ydd_bar.assign(bar.begin() + nq + nv, bar.end());
+            }
+
+            // in2 = [tau; ydd_bar]: (q_bar, yd_bar, tau_bar) by the implicit function theorem, as
+            // forwardDynamicsDerivatives: with mu = H^-1 ydd_bar, tau_bar = mu and x_bar = -mu^T d ID / d x at
+            // ydd = FD(q, yd, tau) - one reverse sweep of the inverse dynamics with placeholder accelerations (input
+            // array 3), which are then replaced by the forward-dynamics expressions; the solve shares the one
+            // factorisation. Contracted with a direction that keeps quaternions unit and implicit clusters on
+            // phi = 0, q_bar equals w^T times the tangent Jacobian of forwardDynamicsDerivatives. Its component
+            // normal to that set (quaternion norm, constraint violation) is the one of -H^-1 d ID / d q: it is not
+            // the derivative of one particular forward-dynamics program off the set. A caller that normalises its
+            // quaternion in its own graph drops that component anyway.
+            void forwardDynamicsVJP(std::vector<Sym> &q_bar, std::vector<Sym> &yd_bar, std::vector<Sym> &tau_bar)
+            {
+                const int nq = m_.getNumPositions(), nv = m_.getNumDegreesOfFreedom();
+                std::vector<Sym> placeholder(nv);
+                for (int i = 0; i < nv; i++)
+                    placeholder[i] = Sym::input(3, i);
+                aux_override_ = &placeholder;
+                const std::vector<Sym> id = inverseDynamics();
+                aux_override_ = nullptr;
+                tau_bar = solveMassMatrix(vjpCotangent());
+                std::vector<Sym> neg_mu(nv);
+                for (int i = 0; i < nv; i++)
+                    neg_mu[i] = -tau_bar[i];
+                std::vector<Sym> wrt = vjpPositions();
+                for (int i = 0; i < nv; i++)
+                    wrt.push_back(inYd(i));
+                std::vector<Sym> bar = adjointSweep(id, neg_mu, wrt);
+                const std::vector<Sym> ydd = forwardDynamicsLTL();
+                std::unordered_map<int32_t, Sym> values;
+                for (int i = 0; i < nv; i++)
+                    values[placeholder[i].id] = ydd[i];
+                bar = substituteInputs(bar, values);
+                q_bar.assign(bar.begin(), bar.begin() + nq);
+                yd_bar.assign(bar.begin() + nq, bar.end());
+            }
+
+            // ---------------------------------------------------------------------------------
             // mass matrix: spanning-tree CRBA + projection H = G^T H_s G   (row-major nv x nv)
             // ---------------------------------------------------------------------------------
             std::vector<Sym> massMatrix()

@@ -33,14 +33,18 @@ namespace grbda
             // dq = tangent-space perturbation of the positions (ModelCompiler::positionTangentMap)
             ALGO_ID_DERIV = 12,    // in: q, yd, ydd     out: dtau/ddq [nv nv], dtau/dyd [nv nv]
             ALGO_FD_DERIV = 13,    // in: q, yd, tau     out: dydd/ddq [nv nv], dydd/dyd [nv nv], dydd/dtau = H^-1 [nv nv]
-            PROGRAM_COUNT = 14
+            // reverse mode (compiled at run time when first used): the cotangent w travels behind the third argument
+            // in input array 2; q_bar is the gradient with respect to the nq stored position entries
+            ALGO_ID_VJP = 14,      // in: q, yd, [ydd; w]  out: q_bar [nq], yd_bar [nv], ydd_bar = H w [nv]
+            ALGO_FD_VJP = 15,      // in: q, yd, [tau; w]  out: q_bar [nq], yd_bar [nv], tau_bar = H^-1 w [nv]
+            PROGRAM_COUNT = 16
         };
         // registry slot a program belongs to
         inline int algoOfProgram(int program) { return program == PROGRAM_FD_LTL ? ALGO_FD : program; }
         inline const char *algoName(int a)
         {
             static const char *names[] = {"id", "fd", "fk", "h", "phi", "gfa", "gfs", "fd_ltl", "contact_kin", "contact_jac",
-                                          "test_force", "osim", "id_deriv", "fd_deriv"};
+                                          "test_force", "osim", "id_deriv", "fd_deriv", "id_vjp", "fd_vjp"};
             return names[a];
         }
 
@@ -111,6 +115,10 @@ namespace grbda
                 break;
             case ALGO_FD_DERIV:
                 n_in[1] = n_in[2] = nv, n_out[0] = n_out[1] = n_out[2] = nv * nv;
+                break;
+            case ALGO_ID_VJP:
+            case ALGO_FD_VJP:
+                n_in[1] = nv, n_in[2] = 2 * nv, n_out[0] = nq, n_out[1] = n_out[2] = nv;
                 break;
             default:
                 throw std::runtime_error("algoSizes: unknown program");
@@ -218,6 +226,18 @@ namespace grbda
                 std::vector<sym::Sym> dq, dyd, dtau;
                 mc.forwardDynamicsDerivatives(dq, dyd, dtau);
                 p.outputs = {dq, dyd, dtau};
+                break;
+            }
+            case ALGO_ID_VJP:
+            case ALGO_FD_VJP:
+            {
+                p.n_in[0] = nq, p.n_in[1] = nv, p.n_in[2] = 2 * nv;
+                std::vector<sym::Sym> q_bar, yd_bar, aux_bar;
+                if (algo == ALGO_ID_VJP)
+                    mc.inverseDynamicsVJP(q_bar, yd_bar, aux_bar);
+                else
+                    mc.forwardDynamicsVJP(q_bar, yd_bar, aux_bar);
+                p.outputs = {q_bar, yd_bar, aux_bar};
                 break;
             }
             default:

@@ -970,6 +970,60 @@ extern "C"
     {
         return launchAlgo(m, compiler::ALGO_FD_DERIV, false, q, yd, tau, dydd_dq, dydd_dyd, dydd_dtau, batch, stream);
     }
+}
+
+namespace
+{
+    // The kernels of the shells read three input arrays per state: the third argument and the cotangent are
+    // packed into [batch][2 nv] (scratch slot 3) with two pitched device-to-device copies on the caller's stream.
+    grbda_status launchVJP(const grbda_model *m, int algo, const double *q, const double *yd, const double *aux,
+                           const double *w, double *q_bar, double *yd_bar, double *aux_bar, int64_t batch, void *stream)
+    {
+        if (!m)
+            return fail(GRBDA_ERR_INVALID_ARGUMENT, "null model");
+        if (m->device < 0 || !m->hasKernels())
+            return fail(GRBDA_ERR_NO_DEVICE, "model was created without a CUDA device (host-only handle)");
+        if (batch < 0)
+            return fail(GRBDA_ERR_INVALID_ARGUMENT, "negative batch");
+        if (grbda_runtime::jitMode() == 0)
+            return fail(GRBDA_ERR_NOT_COMPILED, "vector-Jacobian product programs need run-time compilation (GRBDA_JIT=0)");
+        if (batch == 0)
+            return GRBDA_OK;
+        if (!aux || !w)
+            return fail(GRBDA_ERR_INVALID_ARGUMENT, "null input pointer");
+        DeviceScope scope(m->device);
+        if (scope.error != cudaSuccess)
+            return cudaFail(scope.error, "cudaSetDevice");
+        const size_t row = (size_t)m->model.getNumDegreesOfFreedom() * sizeof(double);
+        double *packed = (double *)m->scratchFor((cudaStream_t)stream, (size_t)batch * 2 * row, 3);
+        if (!packed)
+            return fail(GRBDA_ERR_CUDA, "cannot allocate the packed input buffer: " + m->scratch_error);
+        const size_t nv = row / sizeof(double);
+        cudaError_t e = cudaMemcpy2DAsync(packed, 2 * row, aux, row, row, (size_t)batch, cudaMemcpyDeviceToDevice,
+                                          (cudaStream_t)stream);
+        if (e == cudaSuccess)
+            e = cudaMemcpy2DAsync(packed + nv, 2 * row, w, row, row, (size_t)batch, cudaMemcpyDeviceToDevice,
+                                  (cudaStream_t)stream);
+        if (e != cudaSuccess)
+            return cudaFail(e, "packing the vector-Jacobian product inputs");
+        return launchAlgo(m, algo, false, q, yd, packed, q_bar, yd_bar, aux_bar, batch, stream);
+    }
+} // namespace
+
+extern "C"
+{
+    grbda_status grbda_cuda_inverse_dynamics_vjp_f64(const grbda_model *m, const double *q, const double *yd,
+                                                     const double *ydd, const double *tau_bar, double *q_bar,
+                                                     double *yd_bar, double *ydd_bar, int64_t batch, void *stream)
+    {
+        return launchVJP(m, compiler::ALGO_ID_VJP, q, yd, ydd, tau_bar, q_bar, yd_bar, ydd_bar, batch, stream);
+    }
+    grbda_status grbda_cuda_forward_dynamics_vjp_f64(const grbda_model *m, const double *q, const double *yd,
+                                                     const double *tau, const double *ydd_bar, double *q_bar,
+                                                     double *yd_bar, double *tau_bar, int64_t batch, void *stream)
+    {
+        return launchVJP(m, compiler::ALGO_FD_VJP, q, yd, tau, ydd_bar, q_bar, yd_bar, tau_bar, batch, stream);
+    }
     grbda_status grbda_cuda_inverse_osim_f64(const grbda_model *m, const double *q, double *lambda_inv, int64_t batch,
                                              void *stream)
     {

@@ -154,7 +154,8 @@ grbda_status grbda_cuda_cluster_phi(const grbda_model *m, int cluster, grbda_phi
 /* explicit cluster: G (num_bodies x num_independent, row-major) */
 grbda_status grbda_cuda_cluster_G(const grbda_model *m, int cluster, double *G);
 /* Emitted program of one algorithm (0 ID, 1 FD (articulated-body sweep), 2 FK, 3 H, 4 phi/Kd,
- * 5 / 6 tau_in +/- J^T f_ext, 7 FD as H^-1 (tau - C): cluster CRBA + RNEA bias + branch-sparse L^T D L) written as a binary tape to
+ * 5 / 6 tau_in +/- J^T f_ext, 7 FD as H^-1 (tau - C): cluster CRBA + RNEA bias + branch-sparse L^T D L,
+ * 8-11 operational space, 12 / 13 ID / FD Jacobians, 14 / 15 ID / FD vector-Jacobian products) written as a binary tape to
  * `path` (format: csrc/compiler/compile.h); counts[8] = {nodes, add, mul, div, sqrt, sin, cos,
  * fusable mul+add pairs} of the straight-line program each thread executes. */
 grbda_status grbda_cuda_dump_program(const grbda_model *m, int algo, const char *path, int64_t *counts8);
@@ -265,6 +266,31 @@ grbda_status grbda_cuda_inverse_dynamics_derivatives_f64(const grbda_model *m, c
 grbda_status grbda_cuda_forward_dynamics_derivatives_f64(const grbda_model *m, const double *q, const double *yd,
                                                          const double *tau, double *dydd_dq, double *dydd_dyd,
                                                          double *dydd_dtau, int64_t batch, void *stream);
+
+/* Reverse mode: vector-Jacobian products of the dynamics, what the gradient of a scalar loss of tau or ydd needs
+ * (the torch.autograd functions of the Python package call them). For a cotangent w[batch][nv] of the output:
+ *   inverse dynamics: q_bar = w^T d tau / d q, yd_bar = w^T d tau / d yd, ydd_bar = H w
+ *   forward dynamics: q_bar = w^T d ydd / d q, yd_bar = w^T d ydd / d yd, tau_bar = H^-1 w
+ * One reverse sweep of the model's compiled program per state; the outputs are nq + 2 nv values per state instead
+ * of the 2-3 nv x nv matrices of the Jacobian entry points. q_bar[batch][nq] is the gradient with respect to the
+ * STORED position entries, q_bar[k] = sum_i w_i d out_i / d q[k]:
+ *   inverse dynamics: the exact derivative of the inverse-dynamics program for every entry;
+ *   forward dynamics: contracted with any direction that keeps quaternions unit and implicit clusters on phi = 0,
+ *     it equals w^T times the tangent Jacobian of grbda_cuda_forward_dynamics_derivatives_f64; its component
+ *     normal to that set is the one of -H^-1 d ID / d q (implicit function theorem), not the derivative of one
+ *     particular forward-dynamics kernel off the set.
+ * FP64 only; the programs are compiled at run time when first used. The two per-state input arrays of the third
+ * argument are packed into [batch][2 nv] in a per-stream scratch buffer of the handle with two device-to-device
+ * copies on `stream`, then the kernel runs on `stream`. batch = 0 returns GRBDA_OK without launching anything.
+ * That buffer belongs to the (handle, stream) pair, as the intermediate buffer of the *_ext entry points does: calls
+ * on ONE stream of one handle from several host threads at once are not supported (their copies and kernels may
+ * interleave); give each thread its own stream. */
+grbda_status grbda_cuda_inverse_dynamics_vjp_f64(const grbda_model *m, const double *q, const double *yd,
+                                                 const double *ydd, const double *tau_bar, double *q_bar,
+                                                 double *yd_bar, double *ydd_bar, int64_t batch, void *stream);
+grbda_status grbda_cuda_forward_dynamics_vjp_f64(const grbda_model *m, const double *q, const double *yd,
+                                                 const double *tau, const double *ydd_bar, double *q_bar,
+                                                 double *yd_bar, double *tau_bar, int64_t batch, void *stream);
 
 /* Integration step (semi-implicit Euler): yd_out = yd + dt ydd, q_out = q advanced with yd_out -
  * revolute coordinates q + dt yd; free base p + dt R v_body and ori::integrateQuat(quat, R omega_body,
