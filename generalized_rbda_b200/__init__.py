@@ -33,6 +33,7 @@ ALGO_GFA, ALGO_GFS = 5, 6  # tau_in +/- J^T f_ext (external forces on the termin
 ALGO_CONTACT_KIN, ALGO_CONTACT_JAC, ALGO_TEST_FORCE, ALGO_OSIM = 8, 9, 10, 11  # operational space (contact points)
 ALGO_ID_DERIV, ALGO_FD_DERIV = 12, 13  # derivatives of the dynamics
 ALGO_ID_VJP, ALGO_FD_VJP = 14, 15  # vector-Jacobian products of the dynamics (reverse mode)
+ALGO_GFA_VJP, ALGO_GFS_VJP, ALGO_CONTACT_KIN_VJP = 16, 17, 18  # ... of the external-force programs, contact kinematics
 PROGRAM_FD_LTL = 7  # dump_program only: forward dynamics as CRBA + bias + sparse L^T D L (kernel variant "ltl")
 
 _vp = C.c_void_p
@@ -81,6 +82,9 @@ _lib.grbda_cuda_inverse_dynamics_derivatives_f64.argtypes = [_vp, _vp, _vp, _vp,
 _lib.grbda_cuda_forward_dynamics_derivatives_f64.argtypes = [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _vp]
 _lib.grbda_cuda_inverse_dynamics_vjp_f64.argtypes = [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _vp]
 _lib.grbda_cuda_forward_dynamics_vjp_f64.argtypes = [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _vp]
+_lib.grbda_cuda_inverse_dynamics_ext_vjp_f64.argtypes = [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _vp]
+_lib.grbda_cuda_forward_dynamics_ext_vjp_f64.argtypes = [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _vp]
+_lib.grbda_cuda_contact_kinematics_vjp_f64.argtypes = [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _vp]
 _lib.grbda_cuda_integrate_f64.argtypes = [_vp, _vp, _vp, _vp, C.c_double, _vp, _vp, _vp, _i64, _vp]
 _lib.grbda_cuda_step_f64.argtypes = [_vp, _vp, _vp, _vp, _vp, C.c_double, _vp, _vp, _vp, _i64, _vp]
 _lib.grbda_cuda_dynamics_host_f64.argtypes = [_vp, C.c_int, _vp, _vp, _vp, _vp, _i64]
@@ -105,6 +109,8 @@ EXPORTED_SYMBOLS = [
     "grbda_cuda_inverse_osim_f64",
     "grbda_cuda_inverse_dynamics_derivatives_f64", "grbda_cuda_forward_dynamics_derivatives_f64",
     "grbda_cuda_inverse_dynamics_vjp_f64", "grbda_cuda_forward_dynamics_vjp_f64",
+    "grbda_cuda_inverse_dynamics_ext_vjp_f64", "grbda_cuda_forward_dynamics_ext_vjp_f64",
+    "grbda_cuda_contact_kinematics_vjp_f64",
     "grbda_cuda_inverse_dynamics_f64", "grbda_cuda_inverse_dynamics_f32",
     "grbda_cuda_forward_dynamics_f64", "grbda_cuda_forward_dynamics_f32",
     "grbda_cuda_mass_matrix_f64", "grbda_cuda_mass_matrix_f32",
@@ -203,6 +209,12 @@ def measure_fma_peak(device=0, fp32=False, seconds=0.5):
 
 def _ptr(t):
     return None if t is None else _vp(t.data_ptr())
+
+
+def _rows(t, B, n):
+    """t as B rows (f_ext [B, nf, 6] -> [B, 6 nf]); n is the row length when there are no rows to infer it from.
+    A wrong size is reported by ClusterTreeModel._prep."""
+    return t.reshape(B, -1) if B else t.reshape(0, n)
 
 
 def _stream():
@@ -408,8 +420,7 @@ class ClusterTreeModel:
         in3 = self._prep(in3, self.nv, torch.float64)
         B = q.shape[0]
         nf = len(self.externalForceBodies())
-        f_ext = f_ext.reshape(B, -1)
-        f_ext = self._prep(f_ext, 6 * nf, torch.float64)
+        f_ext = self._prep(_rows(f_ext, B, 6 * nf), 6 * nf, torch.float64)
         if out is None:
             out = torch.empty((B, self.nv), dtype=torch.float64, device=q.device)
         _check(getattr(_lib, name)(self._h, _ptr(q), _ptr(yd), _ptr(in3), _ptr(f_ext), _ptr(out), B, _stream()))
@@ -572,25 +583,51 @@ class ClusterTreeModel:
                                                                 _ptr(dt), q.shape[0], _stream()))
         return dq.transpose(1, 2), dv.transpose(1, 2), dt.transpose(1, 2)
 
-    def _vjp(self, name, q, yd, aux, w):
+    def _vjp(self, dynamics, q, yd, aux, w, f_ext=None):
         import torch
         q = self._prep(q, self.nq, torch.float64)
         yd, aux, w = (self._prep(t, self.nv, torch.float64) for t in (yd, aux, w))
         q_bar = torch.empty_like(q)
         yd_bar, aux_bar = torch.empty_like(yd), torch.empty_like(yd)
-        _check(getattr(_lib, name)(self._h, _ptr(q), _ptr(yd), _ptr(aux), _ptr(w), _ptr(q_bar), _ptr(yd_bar),
-                                   _ptr(aux_bar), q.shape[0], _stream()))
-        return q_bar, yd_bar, aux_bar
+        B = q.shape[0]
+        if f_ext is None:
+            _check(getattr(_lib, "grbda_cuda_%s_vjp_f64" % dynamics)(
+                self._h, _ptr(q), _ptr(yd), _ptr(aux), _ptr(w), _ptr(q_bar), _ptr(yd_bar), _ptr(aux_bar), B, _stream()))
+            return q_bar, yd_bar, aux_bar
+        nf6 = 6 * len(self.externalForceBodies())
+        f = self._prep(_rows(f_ext, B, nf6), nf6, torch.float64)
+        f_bar = torch.empty_like(f)
+        _check(getattr(_lib, "grbda_cuda_%s_ext_vjp_f64" % dynamics)(
+            self._h, _ptr(q), _ptr(yd), _ptr(aux), _ptr(f), _ptr(w), _ptr(q_bar), _ptr(yd_bar), _ptr(aux_bar),
+            _ptr(f_bar), B, _stream()))
+        return q_bar, yd_bar, aux_bar, f_bar.reshape(f_ext.shape)
 
-    def inverseDynamicsVJP(self, q, yd, ydd, tau_bar):
+    def inverseDynamicsVJP(self, q, yd, ydd, tau_bar, f_ext=None):
         """(q_bar[batch, nq], yd_bar[batch, nv], ydd_bar[batch, nv]): the cotangent tau_bar of tau = ID(q, yd, ydd)
-        pulled back to the inputs (ydd_bar = H tau_bar); q_bar is the gradient with respect to the stored positions."""
-        return self._vjp("grbda_cuda_inverse_dynamics_vjp_f64", q, yd, ydd, tau_bar)
+        pulled back to the inputs (ydd_bar = H tau_bar); q_bar is the gradient with respect to the stored positions.
+        With f_ext (as inverseDynamics takes it: tau = ID - J^T f) a fourth tensor, f_bar = -J tau_bar, in the shape
+        of f_ext."""
+        return self._vjp("inverse_dynamics", q, yd, ydd, tau_bar, f_ext)
 
-    def forwardDynamicsVJP(self, q, yd, tau, ydd_bar):
+    def forwardDynamicsVJP(self, q, yd, tau, ydd_bar, f_ext=None):
         """(q_bar[batch, nq], yd_bar[batch, nv], tau_bar[batch, nv]): the cotangent ydd_bar of ydd = FD(q, yd, tau)
-        pulled back to the inputs (tau_bar = H^-1 ydd_bar); q_bar as documented in include/grbda_cuda.h."""
-        return self._vjp("grbda_cuda_forward_dynamics_vjp_f64", q, yd, tau, ydd_bar)
+        pulled back to the inputs (tau_bar = H^-1 ydd_bar); q_bar as documented in include/grbda_cuda.h. With f_ext
+        (ydd = FD(q, yd, tau + J^T f)) a fourth tensor, f_bar = J tau_bar, in the shape of f_ext."""
+        return self._vjp("forward_dynamics", q, yd, tau, ydd_bar, f_ext)
+
+    def contactKinematicsVJP(self, q, yd, p_bar, v_bar):
+        """(q_bar[batch, nq], yd_bar[batch, nv]): the cotangents p_bar / v_bar [batch, n_cp, 3] of contactKinematics
+        pulled back to the inputs (yd_bar = J_lin^T v_bar); q_bar is the gradient with respect to the stored
+        positions."""
+        import torch
+        q = self._prep(q, self.nq, torch.float64)
+        yd = self._prep(yd, self.nv, torch.float64)
+        B = q.shape[0]
+        p_bar, v_bar = (self._prep(_rows(t, B, 3 * self.ncp), 3 * self.ncp, torch.float64) for t in (p_bar, v_bar))
+        q_bar, yd_bar = torch.empty_like(q), torch.empty_like(yd)
+        _check(_lib.grbda_cuda_contact_kinematics_vjp_f64(self._h, _ptr(q), _ptr(yd), _ptr(p_bar), _ptr(v_bar),
+                                                          _ptr(q_bar), _ptr(yd_bar), B, _stream()))
+        return q_bar, yd_bar
 
     def integrate(self, q, yd, ydd, dt, out=None):
         """(q', yd', flags): semi-implicit Euler step, quaternion base by ori::integrateQuat, implicit clusters

@@ -880,12 +880,12 @@ namespace grbda
                     x[k] = Sym::input(IN_Q, k);
                 return x;
             }
-            std::vector<Sym> vjpCotangent() const
+            // the n cotangent entries at input array 2, [first, first + n)
+            std::vector<Sym> vjpCotangent(int n, int first) const
             {
-                const int nv = m_.getNumDegreesOfFreedom();
-                std::vector<Sym> w(nv);
-                for (int i = 0; i < nv; i++)
-                    w[i] = Sym::input(IN_AUX, nv + i);
+                std::vector<Sym> w(n);
+                for (int i = 0; i < n; i++)
+                    w[i] = Sym::input(IN_AUX, first + i);
                 return w;
             }
 
@@ -901,7 +901,7 @@ namespace grbda
                     wrt.push_back(inYd(i));
                 for (int i = 0; i < nv; i++)
                     wrt.push_back(inAux(i));
-                const std::vector<Sym> bar = adjointSweep(tau, vjpCotangent(), wrt);
+                const std::vector<Sym> bar = adjointSweep(tau, vjpCotangent(nv, nv), wrt);
                 q_bar.assign(bar.begin(), bar.begin() + nq);
                 yd_bar.assign(bar.begin() + nq, bar.begin() + nq + nv);
                 ydd_bar.assign(bar.begin() + nq + nv, bar.end());
@@ -925,7 +925,7 @@ namespace grbda
                 aux_override_ = &placeholder;
                 const std::vector<Sym> id = inverseDynamics();
                 aux_override_ = nullptr;
-                tau_bar = solveMassMatrix(vjpCotangent());
+                tau_bar = solveMassMatrix(vjpCotangent(nv, nv));
                 std::vector<Sym> neg_mu(nv);
                 for (int i = 0; i < nv; i++)
                     neg_mu[i] = -tau_bar[i];
@@ -938,6 +938,41 @@ namespace grbda
                 for (int i = 0; i < nv; i++)
                     values[placeholder[i].id] = ydd[i];
                 bar = substituteInputs(bar, values);
+                q_bar.assign(bar.begin(), bar.begin() + nq);
+                yd_bar.assign(bar.begin() + nq, bar.end());
+            }
+
+            // in1 = f_ext [6 nf], in2 = w [nv]: (q_bar, f_bar) of tau_out = tau_in + sign J^T f, one reverse sweep of
+            // generalizedExternalForce. The program is linear in tau_in and in f: tau_in_bar = w (left to the
+            // caller), f_bar = sign J w. The cotangent sits where tau_in does (input array 2, entries 0..nv-1); it
+            // only enters the sweep as the adjoint of the roots. q_bar is the exact derivative of the program for
+            // every stored position entry.
+            void externalForceVJP(int sign, std::vector<Sym> &q_bar, std::vector<Sym> &f_bar)
+            {
+                const int nq = m_.getNumPositions(), nv = m_.getNumDegreesOfFreedom();
+                const int nf = (int)externalForceBodies(m_).size();
+                const std::vector<Sym> tau = generalizedExternalForce(sign);
+                std::vector<Sym> wrt = vjpPositions();
+                for (int k = 0; k < 6 * nf; k++)
+                    wrt.push_back(Sym::input(IN_YD, k));
+                const std::vector<Sym> bar = adjointSweep(tau, vjpCotangent(nv, 0), wrt);
+                q_bar.assign(bar.begin(), bar.begin() + nq);
+                f_bar.assign(bar.begin() + nq, bar.end());
+            }
+
+            // in1 = yd, in2 = [p_bar (3 n_cp); v_bar (3 n_cp)]: (q_bar, yd_bar), one reverse sweep of
+            // contactKinematics. yd_bar = J_lin^T v_bar (the contact velocities are linear in yd); q_bar is the exact
+            // derivative of the program for every stored position entry, as for inverseDynamicsVJP.
+            void contactKinematicsVJP(std::vector<Sym> &q_bar, std::vector<Sym> &yd_bar)
+            {
+                const int nq = m_.getNumPositions(), nv = m_.getNumDegreesOfFreedom();
+                std::vector<Sym> roots, vel;
+                contactKinematics(roots, vel);
+                roots.insert(roots.end(), vel.begin(), vel.end());
+                std::vector<Sym> wrt = vjpPositions();
+                for (int i = 0; i < nv; i++)
+                    wrt.push_back(inYd(i));
+                const std::vector<Sym> bar = adjointSweep(roots, vjpCotangent((int)roots.size(), 0), wrt);
                 q_bar.assign(bar.begin(), bar.begin() + nq);
                 yd_bar.assign(bar.begin() + nq, bar.end());
             }

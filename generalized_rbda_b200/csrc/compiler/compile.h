@@ -37,14 +37,20 @@ namespace grbda
             // in input array 2; q_bar is the gradient with respect to the nq stored position entries
             ALGO_ID_VJP = 14,      // in: q, yd, [ydd; w]  out: q_bar [nq], yd_bar [nv], ydd_bar = H w [nv]
             ALGO_FD_VJP = 15,      // in: q, yd, [tau; w]  out: q_bar [nq], yd_bar [nv], tau_bar = H^-1 w [nv]
-            PROGRAM_COUNT = 16
+            // reverse mode of the external-force programs 5 / 6 (tau_in_bar = w is left to the caller) and of the
+            // contact kinematics 8: the cotangent is input array 2 itself
+            ALGO_GFA_VJP = 16,     // in: q, f_ext [6 nf], w [nv]   out: q_bar [nq], f_bar = J w [6 nf]
+            ALGO_GFS_VJP = 17,     // in: q, f_ext [6 nf], w [nv]   out: q_bar [nq], f_bar = -J w [6 nf]
+            ALGO_CONTACT_KIN_VJP = 18, // in: q, yd, [p_bar; v_bar] [6 n_cp]   out: q_bar [nq], yd_bar = J_lin^T v_bar [nv]
+            PROGRAM_COUNT = 19
         };
         // registry slot a program belongs to
         inline int algoOfProgram(int program) { return program == PROGRAM_FD_LTL ? ALGO_FD : program; }
         inline const char *algoName(int a)
         {
             static const char *names[] = {"id", "fd", "fk", "h", "phi", "gfa", "gfs", "fd_ltl", "contact_kin", "contact_jac",
-                                          "test_force", "osim", "id_deriv", "fd_deriv", "id_vjp", "fd_vjp"};
+                                          "test_force", "osim", "id_deriv", "fd_deriv", "id_vjp", "fd_vjp", "gfa_vjp", "gfs_vjp",
+                                          "contact_kin_vjp"};
             return names[a];
         }
 
@@ -119,6 +125,14 @@ namespace grbda
             case ALGO_ID_VJP:
             case ALGO_FD_VJP:
                 n_in[1] = nv, n_in[2] = 2 * nv, n_out[0] = nq, n_out[1] = n_out[2] = nv;
+                break;
+            case ALGO_GFA_VJP:
+            case ALGO_GFS_VJP:
+                n_in[1] = 6 * (int)ModelCompiler::externalForceBodies(model).size(), n_in[2] = nv;
+                n_out[0] = nq, n_out[1] = n_in[1];
+                break;
+            case ALGO_CONTACT_KIN_VJP:
+                n_in[1] = nv, n_in[2] = 6 * (int)model.contactPoints().size(), n_out[0] = nq, n_out[1] = nv;
                 break;
             default:
                 throw std::runtime_error("algoSizes: unknown program");
@@ -238,6 +252,23 @@ namespace grbda
                 else
                     mc.forwardDynamicsVJP(q_bar, yd_bar, aux_bar);
                 p.outputs = {q_bar, yd_bar, aux_bar};
+                break;
+            }
+            case ALGO_GFA_VJP:
+            case ALGO_GFS_VJP:
+            {
+                p.n_in[0] = nq, p.n_in[1] = 6 * (int)ModelCompiler::externalForceBodies(model).size(), p.n_in[2] = nv;
+                std::vector<sym::Sym> q_bar, f_bar;
+                mc.externalForceVJP(algo == ALGO_GFA_VJP ? 1 : -1, q_bar, f_bar);
+                p.outputs = {q_bar, f_bar};
+                break;
+            }
+            case ALGO_CONTACT_KIN_VJP:
+            {
+                p.n_in[0] = nq, p.n_in[1] = nv, p.n_in[2] = 6 * (int)model.contactPoints().size();
+                std::vector<sym::Sym> q_bar, yd_bar;
+                mc.contactKinematicsVJP(q_bar, yd_bar);
+                p.outputs = {q_bar, yd_bar};
                 break;
             }
             default:

@@ -56,7 +56,9 @@ struct grbda_model
     mutable std::mutex scratch_mutex;
     mutable std::string scratch_error;
     mutable std::map<std::pair<cudaStream_t, int>, Scratch> scratch;
-    // slot 0: tile flags of a launch; slot 1: intermediate generalized forces of the *_ext entry points
+    // slot 0: tile flags of a launch; slot 1: intermediate generalized forces of the *_ext entry points;
+    // slot 2: accelerations of grbda_cuda_step_f64; slot 3: packed inputs of the vector-Jacobian products;
+    // slot 4: the external-force contribution to q_bar of the *_ext_vjp entry points
     unsigned char *scratchFor(cudaStream_t stream, size_t bytes, int slot = 0) const
     {
         std::lock_guard<std::mutex> lock(scratch_mutex);
@@ -925,7 +927,8 @@ extern "C"
             m->model.setContactPoints(pts);
             std::lock_guard<std::mutex> lock(m->jit_ext_mutex);
             if (m->jit_ext)
-                for (int a = compiler::ALGO_CONTACT_KIN; a <= compiler::ALGO_OSIM; a++)
+                for (int a : {compiler::ALGO_CONTACT_KIN, compiler::ALGO_CONTACT_JAC, compiler::ALGO_TEST_FORCE,
+                              compiler::ALGO_OSIM, compiler::ALGO_CONTACT_KIN_VJP})
                     for (int p = 0; p < 2; p++)
                     {
                         if (m->jit_ext->algo[a][p].library)
@@ -974,10 +977,8 @@ extern "C"
 
 namespace
 {
-    // The kernels of the shells read three input arrays per state: the third argument and the cotangent are
-    // packed into [batch][2 nv] (scratch slot 3) with two pitched device-to-device copies on the caller's stream.
-    grbda_status launchVJP(const grbda_model *m, int algo, const double *q, const double *yd, const double *aux,
-                           const double *w, double *q_bar, double *yd_bar, double *aux_bar, int64_t batch, void *stream)
+    // Checks shared by the vector-Jacobian product entry points, before any pointer (batch = 0 launches nothing)
+    grbda_status vjpCheck(const grbda_model *m, int64_t batch)
     {
         if (!m)
             return fail(GRBDA_ERR_INVALID_ARGUMENT, "null model");
@@ -987,26 +988,92 @@ namespace
             return fail(GRBDA_ERR_INVALID_ARGUMENT, "negative batch");
         if (grbda_runtime::jitMode() == 0)
             return fail(GRBDA_ERR_NOT_COMPILED, "vector-Jacobian product programs need run-time compilation (GRBDA_JIT=0)");
-        if (batch == 0)
-            return GRBDA_OK;
+        return GRBDA_OK;
+    }
+
+    // The kernels of the shells read three input arrays per state: two per-state arrays x [batch][nx] and
+    // y [batch][ny] (the third argument and the cotangent, or two cotangents) are packed into [batch][nx + ny]
+    // (scratch slot 3) with two pitched device-to-device copies on the caller's stream.
+    grbda_status packRows(const grbda_model *m, const double *x, size_t nx, const double *y, size_t ny, int64_t batch,
+                          cudaStream_t stream, double *&packed)
+    {
+        const size_t row = (nx + ny) * sizeof(double);
+        packed = (double *)m->scratchFor(stream, (size_t)batch * row, 3);
+        if (!packed)
+            return fail(GRBDA_ERR_CUDA, "cannot allocate the packed input buffer: " + m->scratch_error);
+        cudaError_t e = cudaMemcpy2DAsync(packed, row, x, nx * sizeof(double), nx * sizeof(double), (size_t)batch,
+                                          cudaMemcpyDeviceToDevice, stream);
+        if (e == cudaSuccess)
+            e = cudaMemcpy2DAsync(packed + nx, row, y, ny * sizeof(double), ny * sizeof(double), (size_t)batch,
+                                  cudaMemcpyDeviceToDevice, stream);
+        if (e != cudaSuccess)
+            return cudaFail(e, "packing the vector-Jacobian product inputs");
+        return GRBDA_OK;
+    }
+
+    grbda_status launchVJP(const grbda_model *m, int algo, const double *q, const double *yd, const double *aux,
+                           const double *w, double *q_bar, double *yd_bar, double *aux_bar, int64_t batch, void *stream)
+    {
+        grbda_status st = vjpCheck(m, batch);
+        if (st != GRBDA_OK || batch == 0)
+            return st;
         if (!aux || !w)
             return fail(GRBDA_ERR_INVALID_ARGUMENT, "null input pointer");
         DeviceScope scope(m->device);
         if (scope.error != cudaSuccess)
             return cudaFail(scope.error, "cudaSetDevice");
-        const size_t row = (size_t)m->model.getNumDegreesOfFreedom() * sizeof(double);
-        double *packed = (double *)m->scratchFor((cudaStream_t)stream, (size_t)batch * 2 * row, 3);
-        if (!packed)
-            return fail(GRBDA_ERR_CUDA, "cannot allocate the packed input buffer: " + m->scratch_error);
-        const size_t nv = row / sizeof(double);
-        cudaError_t e = cudaMemcpy2DAsync(packed, 2 * row, aux, row, row, (size_t)batch, cudaMemcpyDeviceToDevice,
-                                          (cudaStream_t)stream);
-        if (e == cudaSuccess)
-            e = cudaMemcpy2DAsync(packed + nv, 2 * row, w, row, row, (size_t)batch, cudaMemcpyDeviceToDevice,
-                                  (cudaStream_t)stream);
-        if (e != cudaSuccess)
-            return cudaFail(e, "packing the vector-Jacobian product inputs");
+        const size_t nv = (size_t)m->model.getNumDegreesOfFreedom();
+        double *packed = nullptr;
+        if ((st = packRows(m, aux, nv, w, nv, batch, (cudaStream_t)stream, packed)) != GRBDA_OK)
+            return st;
         return launchAlgo(m, algo, false, q, yd, packed, q_bar, yd_bar, aux_bar, batch, stream);
+    }
+
+    // The dynamics VJP with external forces, composed of the programs that exist (f_ext != NULL):
+    //   inverse dynamics, tau = ID(q, yd, ydd) - J^T f: ALGO_ID_VJP with w, then ALGO_GFS_VJP(q, f, w);
+    //   forward dynamics, ydd = FD(q, yd, tau'), tau' = tau + J^T f: ALGO_GFA -> tau' (scratch slot 1), ALGO_FD_VJP at
+    //   tau' (tau_bar = H^-1 w), then ALGO_GFA_VJP(q, f, tau_bar).
+    // The force program writes f_bar and its q contribution (scratch slot 4), which one more launch adds to q_bar.
+    grbda_status launchExtVJP(const grbda_model *m, bool forward, const double *q, const double *yd, const double *aux,
+                              const double *f_ext, const double *w, double *q_bar, double *yd_bar, double *aux_bar,
+                              double *f_bar, int64_t batch, void *stream)
+    {
+        grbda_status st = vjpCheck(m, batch);
+        if (st != GRBDA_OK || batch == 0)
+            return st;
+        if (!q || !yd || !aux || !w)
+            return fail(GRBDA_ERR_INVALID_ARGUMENT, "null input pointer");
+        if (!q_bar || !yd_bar || !aux_bar || !f_bar)
+            return fail(GRBDA_ERR_INVALID_ARGUMENT, "null output pointer");
+        DeviceScope scope(m->device);
+        if (scope.error != cudaSuccess)
+            return cudaFail(scope.error, "cudaSetDevice");
+        const cudaStream_t s = (cudaStream_t)stream;
+        const int64_t nq = m->model.getNumPositions(), nv = m->model.getNumDegreesOfFreedom();
+        double *q_gf = (double *)m->scratchFor(s, (size_t)(batch * nq) * sizeof(double), 4);
+        if (!q_gf)
+            return fail(GRBDA_ERR_CUDA, "cannot allocate the external-force q_bar buffer: " + m->scratch_error);
+        if (forward)
+        {
+            double *tau_eff = (double *)m->scratchFor(s, (size_t)(batch * nv) * sizeof(double), 1);
+            if (!tau_eff)
+                return fail(GRBDA_ERR_CUDA, "cannot allocate the intermediate generalized-force buffer: " + m->scratch_error);
+            if ((st = launchAlgo(m, compiler::ALGO_GFA, false, q, f_ext, aux, tau_eff, nullptr, nullptr, batch, stream)) != GRBDA_OK ||
+                (st = launchVJP(m, compiler::ALGO_FD_VJP, q, yd, tau_eff, w, q_bar, yd_bar, aux_bar, batch, stream)) != GRBDA_OK ||
+                (st = launchAlgo(m, compiler::ALGO_GFA_VJP, false, q, f_ext, aux_bar, q_gf, f_bar, nullptr, batch, stream)) != GRBDA_OK)
+                return st;
+        }
+        else if ((st = launchVJP(m, compiler::ALGO_ID_VJP, q, yd, aux, w, q_bar, yd_bar, aux_bar, batch, stream)) != GRBDA_OK ||
+                 (st = launchAlgo(m, compiler::ALGO_GFS_VJP, false, q, f_ext, w, q_gf, f_bar, nullptr, batch, stream)) != GRBDA_OK)
+            return st;
+        const int64_t n = batch * nq;
+        const int grid = (int)std::min<int64_t>((n + 255) / 256, 148 * 8);
+        grbda_kernels::accumulateKernel<<<grid, 256, 0, s>>>(q_bar, q_gf, n);
+        const cudaError_t e = cudaGetLastError();
+        if (e != cudaSuccess)
+            return cudaFail(e, "accumulateKernel");
+        g_launches++;
+        return GRBDA_OK;
     }
 } // namespace
 
@@ -1023,6 +1090,44 @@ extern "C"
                                                      double *yd_bar, double *tau_bar, int64_t batch, void *stream)
     {
         return launchVJP(m, compiler::ALGO_FD_VJP, q, yd, tau, ydd_bar, q_bar, yd_bar, tau_bar, batch, stream);
+    }
+    grbda_status grbda_cuda_inverse_dynamics_ext_vjp_f64(const grbda_model *m, const double *q, const double *yd,
+                                                         const double *ydd, const double *f_ext, const double *tau_bar,
+                                                         double *q_bar, double *yd_bar, double *ydd_bar, double *f_bar,
+                                                         int64_t batch, void *stream)
+    {
+        if (!f_ext)
+            return launchVJP(m, compiler::ALGO_ID_VJP, q, yd, ydd, tau_bar, q_bar, yd_bar, ydd_bar, batch, stream);
+        return launchExtVJP(m, false, q, yd, ydd, f_ext, tau_bar, q_bar, yd_bar, ydd_bar, f_bar, batch, stream);
+    }
+    grbda_status grbda_cuda_forward_dynamics_ext_vjp_f64(const grbda_model *m, const double *q, const double *yd,
+                                                         const double *tau, const double *f_ext, const double *ydd_bar,
+                                                         double *q_bar, double *yd_bar, double *tau_bar, double *f_bar,
+                                                         int64_t batch, void *stream)
+    {
+        if (!f_ext)
+            return launchVJP(m, compiler::ALGO_FD_VJP, q, yd, tau, ydd_bar, q_bar, yd_bar, tau_bar, batch, stream);
+        return launchExtVJP(m, true, q, yd, tau, f_ext, ydd_bar, q_bar, yd_bar, tau_bar, f_bar, batch, stream);
+    }
+    grbda_status grbda_cuda_contact_kinematics_vjp_f64(const grbda_model *m, const double *q, const double *yd,
+                                                       const double *p_bar, const double *v_bar, double *q_bar,
+                                                       double *yd_bar, int64_t batch, void *stream)
+    {
+        if (m && m->model.contactPoints().empty())
+            return fail(GRBDA_ERR_INVALID_ARGUMENT, "the model has no contact points (grbda_cuda_set_contact_points)");
+        grbda_status st = vjpCheck(m, batch);
+        if (st != GRBDA_OK || batch == 0)
+            return st;
+        if (!p_bar || !v_bar)
+            return fail(GRBDA_ERR_INVALID_ARGUMENT, "null input pointer");
+        DeviceScope scope(m->device);
+        if (scope.error != cudaSuccess)
+            return cudaFail(scope.error, "cudaSetDevice");
+        const size_t n = 3 * m->model.contactPoints().size();
+        double *packed = nullptr;
+        if ((st = packRows(m, p_bar, n, v_bar, n, batch, (cudaStream_t)stream, packed)) != GRBDA_OK)
+            return st;
+        return launchAlgo(m, compiler::ALGO_CONTACT_KIN_VJP, false, q, yd, packed, q_bar, yd_bar, nullptr, batch, stream);
     }
     grbda_status grbda_cuda_inverse_osim_f64(const grbda_model *m, const double *q, double *lambda_inv, int64_t batch,
                                              void *stream)

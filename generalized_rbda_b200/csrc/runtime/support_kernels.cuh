@@ -1,5 +1,5 @@
-// Small hand-written support kernels: checksum, row-wise max |x| (constraint violation), FMA peak
-// micro-benchmark (the FP64 / FP32 roofline denominators are measured, not assumed).
+// Small hand-written support kernels: checksum, row-wise max |x| (constraint violation), elementwise
+// accumulation, FMA peak micro-benchmark (the FP64 / FP32 roofline denominators are measured, not assumed).
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -51,6 +51,13 @@ namespace grbda_kernels
         for (int i = 0; i < n; i++)
             m = fmax(m, fabs(x[b * n + i]));
         y[b] = m;
+    }
+
+    // y[i] += x[i]: sums the two contributions to q_bar of the vector-Jacobian products with external forces
+    __global__ void __launch_bounds__(256) accumulateKernel(double *__restrict__ y, const double *__restrict__ x, int64_t n)
+    {
+        for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x)
+            y[i] += x[i];
     }
 
     // Dependent-free FMA streams: 8 independent accumulators per thread, `iters` rounds of 8 FMAs.

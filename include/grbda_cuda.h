@@ -155,7 +155,9 @@ grbda_status grbda_cuda_cluster_phi(const grbda_model *m, int cluster, grbda_phi
 grbda_status grbda_cuda_cluster_G(const grbda_model *m, int cluster, double *G);
 /* Emitted program of one algorithm (0 ID, 1 FD (articulated-body sweep), 2 FK, 3 H, 4 phi/Kd,
  * 5 / 6 tau_in +/- J^T f_ext, 7 FD as H^-1 (tau - C): cluster CRBA + RNEA bias + branch-sparse L^T D L,
- * 8-11 operational space, 12 / 13 ID / FD Jacobians, 14 / 15 ID / FD vector-Jacobian products) written as a binary tape to
+ * 8-11 operational space, 12 / 13 ID / FD Jacobians, 14 / 15 ID / FD vector-Jacobian products, 16 / 17 the
+ * vector-Jacobian products of programs 5 / 6 (in: q, f_ext, w; out: q_bar, f_bar), 18 the one of contact kinematics
+ * (in: q, yd, [p_bar; v_bar]; out: q_bar, yd_bar)) written as a binary tape to
  * `path` (format: csrc/compiler/compile.h); counts[8] = {nodes, add, mul, div, sqrt, sin, cos,
  * fusable mul+add pairs} of the straight-line program each thread executes. */
 grbda_status grbda_cuda_dump_program(const grbda_model *m, int algo, const char *path, int64_t *counts8);
@@ -291,6 +293,36 @@ grbda_status grbda_cuda_inverse_dynamics_vjp_f64(const grbda_model *m, const dou
 grbda_status grbda_cuda_forward_dynamics_vjp_f64(const grbda_model *m, const double *q, const double *yd,
                                                  const double *tau, const double *ydd_bar, double *q_bar,
                                                  double *yd_bar, double *tau_bar, int64_t batch, void *stream);
+/* The same with external forces f_ext[batch][nf][6] on grbda_cuda_external_force_bodies (as the *_ext entry points
+ * take them); f_bar[batch][nf][6] receives their cotangent. f_ext = NULL means no external forces: the call is then
+ * exactly the VJP above and f_bar is not written (it may be NULL).
+ *   inverse dynamics, tau = ID(q, yd, ydd) - J^T f: q_bar, yd_bar, ydd_bar = H tau_bar as above, f_bar = -J tau_bar.
+ *     Launches: the ID VJP (two copies + one kernel), the program of -J^T f reversed (q contribution to a per-stream
+ *     scratch buffer of nq doubles per state), one elementwise kernel that adds it to q_bar.
+ *   forward dynamics, ydd = FD(q, yd, tau + J^T f): tau_bar = H^-1 ydd_bar, f_bar = J tau_bar. Launches: tau + J^T f
+ *     into a scratch buffer (what grbda_cuda_forward_dynamics_ext_f64 runs), the FD VJP at that torque (two copies +
+ *     one kernel), the program of J^T f reversed with tau_bar, one elementwise kernel that adds its q contribution.
+ * q_bar: the external-force part is the exact derivative of the program J(q)^T f for every stored position entry;
+ * the dynamics part means what it means above (exact for ID; for FD the manifold convention above, at tau + J^T f).
+ * The scratch buffers and the concurrency caveat are those of the VJP entry points above. */
+grbda_status grbda_cuda_inverse_dynamics_ext_vjp_f64(const grbda_model *m, const double *q, const double *yd,
+                                                     const double *ydd, const double *f_ext, const double *tau_bar,
+                                                     double *q_bar, double *yd_bar, double *ydd_bar, double *f_bar,
+                                                     int64_t batch, void *stream);
+grbda_status grbda_cuda_forward_dynamics_ext_vjp_f64(const grbda_model *m, const double *q, const double *yd,
+                                                     const double *tau, const double *f_ext, const double *ydd_bar,
+                                                     double *q_bar, double *yd_bar, double *tau_bar, double *f_bar,
+                                                     int64_t batch, void *stream);
+/* Reverse mode of grbda_cuda_contact_kinematics_f64: for cotangents p_bar[batch][n_cp][3] and v_bar[batch][n_cp][3]
+ * of the contact positions and velocities, yd_bar[batch][nv] = J_lin^T v_bar (J_lin: the linear rows of the contact
+ * Jacobians) and q_bar[batch][nq], the exact derivative of the contact-kinematics program for every stored position
+ * entry (as for the inverse dynamics). p_bar and v_bar are packed into [batch][6 n_cp] in the per-stream scratch
+ * buffer of the VJP entry points (two copies), then one kernel runs; same concurrency caveat. The program is
+ * specialised for the contact set and compiled at run time when first used; a model without contact points is
+ * refused as by grbda_cuda_contact_kinematics_f64. */
+grbda_status grbda_cuda_contact_kinematics_vjp_f64(const grbda_model *m, const double *q, const double *yd,
+                                                   const double *p_bar, const double *v_bar, double *q_bar,
+                                                   double *yd_bar, int64_t batch, void *stream);
 
 /* Integration step (semi-implicit Euler): yd_out = yd + dt ydd, q_out = q advanced with yd_out -
  * revolute coordinates q + dt yd; free base p + dt R v_body and ori::integrateQuat(quat, R omega_body,

@@ -4,7 +4,14 @@ inverse dynamics is timed without H w (it would need the mass-matrix kernel and 
 bound. Each record names the card and its power limit, read in the same run, and gives the operation counts of the
 programs and, for the VJP kernels, the launch shape and the registers / stack (local memory) per thread that
 cuobjdump -res-usage reports for the cubin (the largest over the kernels of the cubin).
-Usage: python tools/vjp_timing.py > profiles/r3_vjp.jsonl"""
+
+--ext-contact: the vector-Jacobian products with external forces and of the contact kinematics instead, 2^20 states of
+TelloWithArms (default force bodies), Mini Cheetah and MIT humanoid with the contact set of the tests: the forward
+entry points, their VJPs, and for the contact kinematics the route contactJacobians + einsum (yd_bar = J_lin^T v_bar
+only) at the largest batch of 2^20, 2^19, ... whose J fits in half the free memory. No Jacobian entry point takes
+external forces, so the dynamics with forces have no Jacobian route.
+Usage: python tools/vjp_timing.py > profiles/r3_vjp.jsonl
+       python tools/vjp_timing.py --ext-contact > profiles/r4_ext_contact_vjp.jsonl"""
 import json
 import os
 import re
@@ -71,7 +78,66 @@ def first_call(fn):
     return round(time.time() - t0, 2)
 
 
+def ext_contact(gpu_name, power_limit):
+    sys.path.insert(0, os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests"))
+    from test_compiler_cpu import contact_set
+    for robot in ("tello_with_arms", "mini_cheetah", "mit_humanoid"):
+        m = grbda.ClusterTreeModel.from_robot(robot)
+        bodies, offsets, ee = contact_set(m)
+        m.setContactPoints(bodies, offsets, ee)
+        nf = len(m.externalForceBodies())
+        rec = {"model": robot, "nq": m.nq, "nv": m.nv, "force_bodies": nf, "contact_points": m.ncp,
+               "gpu": gpu_name, "power_limit": power_limit}
+        rec.update({k + "_flops": m.dump_program(a)["flops"] for k, a in (
+            ("gfa", grbda.ALGO_GFA), ("gfs", grbda.ALGO_GFS), ("gfa_vjp", grbda.ALGO_GFA_VJP),
+            ("gfs_vjp", grbda.ALGO_GFS_VJP), ("contact_kin", grbda.ALGO_CONTACT_KIN),
+            ("contact_jac", grbda.ALGO_CONTACT_JAC), ("contact_kin_vjp", grbda.ALGO_CONTACT_KIN_VJP))})
+        q, yd, aux, _ = m.generateStates(128)
+        w, f = torch.rand_like(aux), torch.rand(128, nf, 6, dtype=torch.float64, device=q.device)
+        rec["id_ext_vjp_first_call_s"] = first_call(lambda: m.inverseDynamicsVJP(q, yd, aux, w, f_ext=f))
+        rec["fd_ext_vjp_first_call_s"] = first_call(lambda: m.forwardDynamicsVJP(q, yd, aux, w, f_ext=f))
+        p_bar = torch.rand(128, m.ncp, 3, dtype=torch.float64, device=q.device)
+        rec["contact_kin_vjp_first_call_s"] = first_call(lambda: m.contactKinematicsVJP(q, yd, p_bar, p_bar))
+        for name, algo in (("gfa_vjp", grbda.ALGO_GFA_VJP), ("gfs_vjp", grbda.ALGO_GFS_VJP),
+                           ("contact_kin_vjp", grbda.ALGO_CONTACT_KIN_VJP)):
+            rec[name + "_nvrtc_ms"] = m.kernel_info(algo)["compile_ms"]
+            rec.update({name + "_" + k: v for k, v in resources(m, algo).items()})
+        B = 1 << 20
+        rec["states"] = B
+        q, yd, aux, _ = m.generateStates(B)
+        w = torch.rand_like(aux) * 2 - 1
+        f = torch.rand(B, nf, 6, dtype=torch.float64, device=q.device) * 40 - 20
+        out = torch.empty_like(aux)
+        rec["id_ext_ms"] = round(timeit(lambda: m.inverseDynamics(q, yd, aux, out=out, f_ext=f)), 4)
+        rec["fd_ext_ms"] = round(timeit(lambda: m.forwardDynamics(q, yd, aux, out=out, f_ext=f)), 4)
+        rec["id_ext_vjp_ms"] = round(timeit(lambda: m.inverseDynamicsVJP(q, yd, aux, w, f_ext=f)), 4)
+        rec["fd_ext_vjp_ms"] = round(timeit(lambda: m.forwardDynamicsVJP(q, yd, aux, w, f_ext=f)), 4)
+        rec["id_vjp_ms"] = round(timeit(lambda: m.inverseDynamicsVJP(q, yd, aux, w)), 4)
+        rec["fd_vjp_ms"] = round(timeit(lambda: m.forwardDynamicsVJP(q, yd, aux, w)), 4)
+        del aux, w, f, out
+        p_bar = torch.rand(B, m.ncp, 3, dtype=torch.float64, device=q.device) * 2 - 1
+        v_bar = torch.rand_like(p_bar) * 2 - 1
+        rec["contact_kin_ms"] = round(timeit(lambda: m.contactKinematics(q, yd)), 4)
+        rec["contact_kin_vjp_ms"] = round(timeit(lambda: m.contactKinematicsVJP(q, yd, p_bar, v_bar)), 4)
+        Bj = B
+        while Bj * m.ncp * 6 * m.nv * 8 > torch.cuda.mem_get_info()[0] // 2:
+            Bj //= 2
+        qj, vj = q[:Bj], v_bar[:Bj]
+        rec["contact_jacobian_route_states"] = Bj
+        rec["contact_jacobian_route_ms"] = round(timeit(
+            lambda: torch.einsum("bci,bcik->bk", vj, m.contactJacobians(qj)[:, :, 3:, :])), 4)
+        rec["contact_kin_vjp_ms_at_route_states"] = round(timeit(
+            lambda: m.contactKinematicsVJP(qj, yd[:Bj], p_bar[:Bj], vj)), 4)
+        print(json.dumps(rec), flush=True)
+        del q, yd, p_bar, v_bar, qj, vj
+        torch.cuda.empty_cache()
+
+
 gpu_name, power_limit = card()
+if "--ext-contact" in sys.argv:
+    ext_contact(gpu_name, power_limit)
+    WORK.cleanup()
+    sys.exit(0)
 for robot in ROBOTS:
     m = grbda.ClusterTreeModel.from_robot(robot)
     flops = {k: m.dump_program(a)["flops"] for k, a in (("id", grbda.ALGO_ID), ("fd_ltl", grbda.PROGRAM_FD_LTL),
