@@ -631,7 +631,8 @@ class ClusterTreeModel:
 
     def integrate(self, q, yd, ydd, dt, out=None):
         """(q', yd', flags): semi-implicit Euler step, quaternion base by ori::integrateQuat, implicit clusters
-        projected back onto phi = 0; flags[b] = 1 where that projection failed."""
+        projected back onto phi = 0; flags[b] = 1 where that projection failed. A roll-pitch-yaw base is refused:
+        flags = 1 for every state and the base positions are copied unchanged (include/grbda_cuda.h)."""
         import torch
         q = self._prep(q, self.nq, torch.float64)
         yd, ydd = self._prep(yd, self.nv, torch.float64), self._prep(ydd, self.nv, torch.float64)

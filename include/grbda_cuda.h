@@ -329,7 +329,9 @@ grbda_status grbda_cuda_contact_kinematics_vjp_f64(const grbda_model *m, const d
  * dt) (include/grbda/Utils/OrientationTools.h:387-413); clusters with an implicit loop constraint
  * advance their independent coordinates and are projected back onto phi(q) = 0 (Newton on the
  * dependent coordinates, the iteration of GenericJoint.cpp:290-385). flags (optional, int32 per
- * state): 1 where the projection did not converge. q_out / yd_out may alias q / yd. */
+ * state): 1 where the projection did not converge. A roll-pitch-yaw free base (GRBDA_CLUSTER_FREE_RPY) has no
+ * integration rule and is refused per state: flags = 1 for every state, its six positions are copied unchanged to
+ * q_out, the other clusters advance as above, and yd_out still holds yd + dt ydd. q_out / yd_out may alias q / yd. */
 grbda_status grbda_cuda_integrate_f64(const grbda_model *m, const double *q, const double *yd, const double *ydd,
                                       double dt, double *q_out, double *yd_out, int32_t *flags, int64_t batch,
                                       void *stream);
