@@ -35,6 +35,7 @@ ALGO_ID_DERIV, ALGO_FD_DERIV = 12, 13  # derivatives of the dynamics
 ALGO_ID_VJP, ALGO_FD_VJP = 14, 15  # vector-Jacobian products of the dynamics (reverse mode)
 ALGO_GFA_VJP, ALGO_GFS_VJP, ALGO_CONTACT_KIN_VJP = 16, 17, 18  # ... of the external-force programs, contact kinematics
 PROGRAM_FD_LTL = 7  # dump_program only: forward dynamics as CRBA + bias + sparse L^T D L (kernel variant "ltl")
+PROGRAM_INTEGRATE_VJP = -2  # prepare / jit_compile: the reverse integration step (GRBDA_PROGRAM_INTEGRATE_VJP)
 
 _vp = C.c_void_p
 _i64 = C.c_int64
@@ -87,6 +88,9 @@ _lib.grbda_cuda_forward_dynamics_ext_vjp_f64.argtypes = [_vp, _vp, _vp, _vp, _vp
 _lib.grbda_cuda_contact_kinematics_vjp_f64.argtypes = [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _vp]
 _lib.grbda_cuda_integrate_f64.argtypes = [_vp, _vp, _vp, _vp, C.c_double, _vp, _vp, _vp, _i64, _vp]
 _lib.grbda_cuda_step_f64.argtypes = [_vp, _vp, _vp, _vp, _vp, C.c_double, _vp, _vp, _vp, _i64, _vp]
+_lib.grbda_cuda_integrate_vjp_f64.argtypes = [_vp, _vp, _vp, _vp, C.c_double, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _vp]
+_lib.grbda_cuda_step_vjp_f64.argtypes = [_vp, _vp, _vp, _vp, _vp, C.c_double, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64,
+                                         _vp]
 _lib.grbda_cuda_dynamics_host_f64.argtypes = [_vp, C.c_int, _vp, _vp, _vp, _vp, _i64]
 _lib.grbda_cuda_forward_inverse_host_f64.argtypes = [_vp, _vp, _vp, _vp, _vp, _vp, _i64]
 _lib.grbda_cuda_bind_host_to_device.argtypes = [C.c_int, _vp]
@@ -103,7 +107,8 @@ EXPORTED_SYMBOLS = [
     "grbda_cuda_cluster_G", "grbda_cuda_model_gravity", "grbda_cuda_cluster_phi", "grbda_cuda_dump_program", "grbda_cuda_kernel_counts", "grbda_cuda_emit_source",
     "grbda_cuda_model_prepare", "grbda_cuda_kernel_info", "grbda_cuda_jit_compile",
     "grbda_cuda_external_force_bodies", "grbda_cuda_inverse_dynamics_ext_f64", "grbda_cuda_forward_dynamics_ext_f64",
-    "grbda_cuda_integrate_f64", "grbda_cuda_step_f64", "grbda_cuda_set_external_force_bodies",
+    "grbda_cuda_integrate_f64", "grbda_cuda_step_f64", "grbda_cuda_integrate_vjp_f64", "grbda_cuda_step_vjp_f64",
+    "grbda_cuda_set_external_force_bodies",
     "grbda_cuda_set_contact_points", "grbda_cuda_num_contact_points", "grbda_cuda_num_end_effectors",
     "grbda_cuda_contact_kinematics_f64", "grbda_cuda_contact_jacobians_f64", "grbda_cuda_apply_test_force_f64",
     "grbda_cuda_inverse_osim_f64",
@@ -454,7 +459,8 @@ class ClusterTreeModel:
                     compile_ms=v[6], ready=bool(v[7]))
 
     def jit_compile(self, algo, f32=False, source_path=None, cubin_path=None):
-        """Run-time compiler without a device: CUDA text and / or NVRTC cubin of one entry point (algo -1: generator)."""
+        """Run-time compiler without a device: CUDA text and / or NVRTC cubin of one entry point (algo -1: generator,
+        PROGRAM_INTEGRATE_VJP: the reverse integration step)."""
         _check(_lib.grbda_cuda_jit_compile(self._h, algo, int(bool(f32)),
                                            source_path.encode() if source_path else None,
                                            cubin_path.encode() if cubin_path else None))
@@ -655,6 +661,42 @@ class ClusterTreeModel:
         _check(_lib.grbda_cuda_step_f64(self._h, _ptr(q), _ptr(yd), _ptr(tau), _ptr(f_ext), float(dt), _ptr(qo),
                                         _ptr(ydo), _ptr(flags), B, _stream()))
         return qo, ydo, flags
+
+    def integrateVJP(self, q, yd, ydd, dt, q_out_bar, yd_out_bar):
+        """(q_bar[batch, nq], yd_bar[batch, nv], ydd_bar[batch, nv], flags[batch]): the cotangents of (q', yd') =
+        integrate(q, yd, ydd, dt) pulled back to the inputs; q_bar is the exact derivative of the step for every stored
+        position entry, flags those of integrate (values of flagged states are meaningless; include/grbda_cuda.h)."""
+        import torch
+        q, q_out_bar = (self._prep(t, self.nq, torch.float64) for t in (q, q_out_bar))
+        yd, ydd, yd_out_bar = (self._prep(t, self.nv, torch.float64) for t in (yd, ydd, yd_out_bar))
+        q_bar, yd_bar, ydd_bar = torch.empty_like(q), torch.empty_like(yd), torch.empty_like(yd)
+        flags = torch.empty((q.shape[0],), dtype=torch.int32, device=q.device)
+        _check(_lib.grbda_cuda_integrate_vjp_f64(self._h, _ptr(q), _ptr(yd), _ptr(ydd), float(dt), _ptr(q_out_bar),
+                                                 _ptr(yd_out_bar), _ptr(q_bar), _ptr(yd_bar), _ptr(ydd_bar), _ptr(flags),
+                                                 q.shape[0], _stream()))
+        return q_bar, yd_bar, ydd_bar, flags
+
+    def stepVJP(self, q, yd, tau, dt, q_out_bar, yd_out_bar, f_ext=None):
+        """(q_bar, yd_bar, tau_bar[, f_bar], flags): the cotangents of (q', yd') = step(q, yd, tau, dt, f_ext) pulled
+        back to the inputs; f_bar (with f_ext only) has the shape of f_ext. The integration part of q_bar is exact, the
+        dynamics part keeps the convention of forwardDynamicsVJP (include/grbda_cuda.h)."""
+        import torch
+        q, q_out_bar = (self._prep(t, self.nq, torch.float64) for t in (q, q_out_bar))
+        yd, tau, yd_out_bar = (self._prep(t, self.nv, torch.float64) for t in (yd, tau, yd_out_bar))
+        B = q.shape[0]
+        f = f_bar = None
+        if f_ext is not None:
+            nf6 = 6 * len(self.externalForceBodies())
+            f = self._prep(_rows(f_ext, B, nf6), nf6, torch.float64)
+            f_bar = torch.empty_like(f)
+        q_bar, yd_bar, tau_bar = torch.empty_like(q), torch.empty_like(yd), torch.empty_like(yd)
+        flags = torch.empty((B,), dtype=torch.int32, device=q.device)
+        _check(_lib.grbda_cuda_step_vjp_f64(self._h, _ptr(q), _ptr(yd), _ptr(tau), _ptr(f), float(dt), _ptr(q_out_bar),
+                                            _ptr(yd_out_bar), _ptr(q_bar), _ptr(yd_bar), _ptr(tau_bar), _ptr(f_bar),
+                                            _ptr(flags), B, _stream()))
+        if f_ext is None:
+            return q_bar, yd_bar, tau_bar, flags
+        return q_bar, yd_bar, tau_bar, f_bar.reshape(f_ext.shape), flags
 
     def getMassMatrix(self, q, out=None):
         """H[batch, nv, nv]   (ClusterTreeModel::getMassMatrix)"""

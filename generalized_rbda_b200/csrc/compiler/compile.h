@@ -414,6 +414,63 @@ namespace grbda
         }
 
 
+        // `struct Cluster<index>` of one implicit cluster (kernels/stategen.cuh): N, NC, ind(), dep() and the (phi, K_d)
+        // evaluator the Newton projection uses. with_jacobian adds jacobian(q, Kd, Ki), K_d and K_ind of the same
+        // implicitJacobian, for the reverse integration step.
+        inline void emitClusterEvaluator(std::ostream &os, const ClusterTreeModel &model, const ClusterTreeNode &c,
+                                         bool with_jacobian)
+        {
+            const ClusterDesc &d = c.joint_;
+            std::vector<int> ind, dep;
+            for (int i = 0; i < d.num_bodies; i++)
+                (d.independent[i] ? ind : dep).push_back(i);
+            // the body of one function of q: outputs(phi, K_d, K_ind) picks its output arrays
+            auto body = [&](auto outputs) {
+                sym::Graph graph;
+                sym::GraphScope scope(graph);
+                ModelCompiler mc(model);
+                std::vector<sym::Sym> q(d.num_bodies), phi, K, Kd, Ki;
+                for (int i = 0; i < d.num_bodies; i++)
+                    q[i] = sym::Sym::input(0, i);
+                mc.implicitJacobian(d, q, nullptr, phi, K, nullptr);
+                for (int i = 0; i < d.num_constraints; i++)
+                {
+                    for (int j : dep)
+                        Kd.push_back(K[i * d.num_bodies + j]);
+                    for (int j : ind)
+                        Ki.push_back(K[i * d.num_bodies + j]);
+                }
+                Program p;
+                p.outputs = outputs(phi, Kd, Ki);
+                return Emitter(graph, p).cudaBody();
+            };
+            os << "struct Cluster" << c.index_ << "\n{\n    static constexpr int N = " << d.num_bodies
+               << ", NC = " << d.num_constraints << ";\n";
+            os << "    static __device__ __forceinline__ int ind(int i) { const int t[] = {";
+            for (size_t i = 0; i < ind.size(); i++)
+                os << ind[i] << (i + 1 < ind.size() ? ", " : "");
+            os << "}; return t[i]; }\n";
+            os << "    static __device__ __forceinline__ int dep(int i) { const int t[] = {";
+            for (size_t i = 0; i < dep.size(); i++)
+                os << dep[i] << (i + 1 < dep.size() ? ", " : "");
+            os << "}; return t[i]; }\n";
+            const char *prologue = "        typedef double real;\n        constexpr bool FAST = false;\n"
+                                   "#define KC(x) ((real)(x))\n#define GRBDA_PIN(x, late) (x)\n#define GRBDA_DIV(a, b) ((a) / (b))\n#define IN0(i) q[i]\n";
+            const char *epilogue = "#undef KC\n#undef KT\n#undef GRBDA_PIN\n#undef GRBDA_DIV\n#undef IN0\n#undef OUT0\n#undef OUT1\n    }\n";
+            os << "    static __device__ __noinline__ void eval(const double *q, double *phi, double *Kd)\n    {\n" << prologue
+               << "#define OUT0(i, x) phi[i] = (x)\n#define OUT1(i, x) Kd[i] = (x)\n";
+            os << body([](auto &phi, auto &Kd, auto &) { return std::vector<std::vector<sym::Sym>>{phi, Kd}; });
+            os << epilogue;
+            if (with_jacobian)
+            {
+                os << "    static __device__ __noinline__ void jacobian(const double *q, double *Kd, double *Ki)\n    {\n"
+                   << prologue << "#define OUT0(i, x) Kd[i] = (x)\n#define OUT1(i, x) Ki[i] = (x)\n";
+                os << body([](auto &, auto &Kd, auto &Ki) { return std::vector<std::vector<sym::Sym>>{Kd, Ki}; });
+                os << epilogue;
+            }
+            os << "};\n\n";
+        }
+
         // State generator of one model (kernels/stategen.cuh): one (phi, K_d) evaluator per implicit cluster and
         // `struct Gen` that fills one random valid state. Shared by tools/modelc.cpp and the run-time compiler.
         inline void emitGenerator(std::ostream &os, const ClusterTreeModel &model)
@@ -421,43 +478,8 @@ namespace grbda
             const int nq = model.getNumPositions(), nv = model.getNumDegreesOfFreedom();
             // one (phi, Kd) evaluator per implicit cluster
             for (const ClusterTreeNode &c : model.clusters())
-            {
-                if (c.joint_.type != ClusterType::Implicit)
-                    continue;
-                const ClusterDesc &d = c.joint_;
-                sym::Graph graph;
-                sym::GraphScope scope(graph);
-                ModelCompiler mc(model);
-                std::vector<sym::Sym> q(d.num_bodies), phi, K, Kd;
-                for (int i = 0; i < d.num_bodies; i++)
-                    q[i] = sym::Sym::input(0, i);
-                mc.implicitJacobian(d, q, nullptr, phi, K, nullptr);
-                std::vector<int> ind, dep;
-                for (int i = 0; i < d.num_bodies; i++)
-                    (d.independent[i] ? ind : dep).push_back(i);
-                for (int i = 0; i < d.num_constraints; i++)
-                    for (int j : dep)
-                        Kd.push_back(K[i * d.num_bodies + j]);
-                Program p;
-                p.outputs = {phi, Kd};
-                Emitter em(graph, p);
-                os << "struct Cluster" << c.index_ << "\n{\n    static constexpr int N = " << d.num_bodies
-                   << ", NC = " << d.num_constraints << ";\n";
-                os << "    static __device__ __forceinline__ int ind(int i) { const int t[] = {";
-                for (size_t i = 0; i < ind.size(); i++)
-                    os << ind[i] << (i + 1 < ind.size() ? ", " : "");
-                os << "}; return t[i]; }\n";
-                os << "    static __device__ __forceinline__ int dep(int i) { const int t[] = {";
-                for (size_t i = 0; i < dep.size(); i++)
-                    os << dep[i] << (i + 1 < dep.size() ? ", " : "");
-                os << "}; return t[i]; }\n";
-                os << "    static __device__ __noinline__ void eval(const double *q, double *phi, double *Kd)\n    {\n"
-                      "        typedef double real;\n        constexpr bool FAST = false;\n"
-                      "#define KC(x) ((real)(x))\n#define GRBDA_PIN(x, late) (x)\n#define GRBDA_DIV(a, b) ((a) / (b))\n#define IN0(i) q[i]\n#define OUT0(i, x) phi[i] = (x)\n"
-                      "#define OUT1(i, x) Kd[i] = (x)\n";
-                os << em.cudaBody();
-                os << "#undef KC\n#undef KT\n#undef GRBDA_PIN\n#undef GRBDA_DIV\n#undef IN0\n#undef OUT0\n#undef OUT1\n    }\n};\n\n";
-            }
+                if (c.joint_.type == ClusterType::Implicit)
+                    emitClusterEvaluator(os, model, c, false);
             os << "struct Gen\n{\n    static constexpr int NQ = " << nq << ", NV = " << nv << ";\n";
             os << "    static __device__ bool run(Philox &rng, double *q, double *yd, double *aux)\n    {\n"
                   "        bool ok = true;\n";
@@ -508,6 +530,49 @@ namespace grbda
                         if (d.independent[i])
                             os << "        qn[" << pi + i << "] += dt * yd[" << vi + k++ << "];\n";
                     os << "        ok = projectImplicitPosition<Cluster" << c.index_ << ">(qn + " << pi << ") && ok;\n";
+                }
+            }
+            os << "        return ok;\n    }\n};\n";
+        }
+
+        // Reverse mode of `struct Step` (kernels/stategen.cuh integrateVjpState): one evaluator per implicit cluster
+        // with K_ind, and `struct StepVjp` whose run(q, yd_new, dt, q_out_bar, q_bar, v_bar) re-runs the step cluster by
+        // cluster, writes q_bar and adds the positions' part to v_bar. Compiled at run time for every model.
+        inline void emitIntegrateVjp(std::ostream &os, const ClusterTreeModel &model)
+        {
+            for (const ClusterTreeNode &c : model.clusters())
+                if (c.joint_.type == ClusterType::Implicit)
+                    emitClusterEvaluator(os, model, c, true);
+            os << "struct StepVjp\n{\n    static constexpr int NQ = " << model.getNumPositions()
+               << ", NV = " << model.getNumDegreesOfFreedom() << ";\n";
+            os << "    static __device__ bool run(const double *q, const double *yd, double dt, const double *q_out_bar,\n"
+                  "                               double *q_bar, double *v_bar)\n    {\n        bool ok = true;\n";
+            for (const ClusterTreeNode &c : model.clusters())
+            {
+                const ClusterDesc &d = c.joint_;
+                const int pi = c.position_index_, vi = c.velocity_index_;
+                if (d.type == ClusterType::FreeQuaternion)
+                    os << "        integrateFreeQuaternionVjp(q + " << pi << ", yd + " << vi << ", dt, q_out_bar + " << pi
+                       << ", q_bar + " << pi << ", v_bar + " << vi << ");\n";
+                else if (d.type == ClusterType::FreeRollPitchYaw) // the step copies the positions and flags the state
+                    os << "        for (int i = 0; i < 6; i++) q_bar[" << pi << " + i] = q_out_bar[" << pi
+                       << " + i];\n        ok = false;\n";
+                else if (d.type == ClusterType::Explicit)
+                    os << "        for (int i = 0; i < " << d.num_positions << "; i++)\n        {\n            q_bar[" << pi
+                       << " + i] = q_out_bar[" << pi << " + i];\n            v_bar[" << vi << " + i] += dt * q_out_bar["
+                       << pi << " + i];\n        }\n";
+                else
+                {
+                    // the primal's projection, then the adjoint at the point it converged to
+                    os << "        {\n            double qn[" << d.num_bodies << "];\n            for (int i = 0; i < "
+                       << d.num_bodies << "; i++) qn[i] = q[" << pi << " + i];\n";
+                    int k = 0;
+                    for (int i = 0; i < d.num_bodies; i++)
+                        if (d.independent[i])
+                            os << "            qn[" << i << "] += dt * yd[" << vi + k++ << "];\n";
+                    os << "            ok = projectImplicitPosition<Cluster" << c.index_ << ">(qn) && ok;\n"
+                       << "            implicitPositionVjp<Cluster" << c.index_ << ">(qn, dt, q_out_bar + " << pi
+                       << ", q_bar + " << pi << ", v_bar + " << vi << ");\n        }\n";
                 }
             }
             os << "        return ok;\n    }\n};\n";

@@ -313,6 +313,187 @@ namespace grbda_kernels
         return sqrt(s) < 1e-10;
     }
 
+    // ---- reverse mode of the integration step -------------------------------------------------------------
+    // The adjoints re-run the primal of their cluster and pull the cotangent q_out_bar of its new positions back:
+    // q_bar (written) is the exact derivative of what the step computes for every stored position entry, yd_bar
+    // (accumulated) is the part that reaches the new velocities through the positions.
+
+    // Free joint (integrateFreeQuaternion): p' = p + dt R(quat) v_b, quat' = normalise(d(R(quat) w_b) (x) quat) with
+    // the increment d(omega) = (cos(a t), sin(a t) / t omega), a = dt / 2, t = |omega|. R is the polynomial of the raw
+    // stored entries, so a quaternion off the unit sphere gets the derivative of exactly that polynomial. Jacobian of d:
+    //   d d0 / d omega = -a S omega^T,   d dvec / d omega = S I + c2 omega omega^T,
+    //   S = sin(a t) / t,   c2 = (a cos(a t) - S) / t^2.
+    // Below a t = 1e-2 both are Taylor series (S = a - a^3 t^2 / 6 + ..., c2 = -a^3 / 3 + a^5 t^2 / 30 - ...), so the
+    // adjoint is finite and continuous at rest, where the primal takes d = (1, 0, 0, 0). At the switch the series
+    // are exact to rounding; the closed form of c2 loses ~3e-12 of itself to cancellation there, but c2 enters
+    // multiplied by t^2, i.e. ~3e-16 relative to S.
+    __device__ inline void integrateFreeQuaternionVjp(const double *q, const double *yd, double dt, const double *q_out_bar,
+                                                      double *q_bar, double *yd_bar)
+    {
+        const double w = q[3], x = q[4], y = q[5], z = q[6];
+        const double R[9] = {1 - 2 * (y * y + z * z), 2 * (x * y - w * z), 2 * (x * z + w * y),
+                             2 * (x * y + w * z), 1 - 2 * (x * x + z * z), 2 * (y * z - w * x),
+                             2 * (x * z - w * y), 2 * (y * z + w * x), 1 - 2 * (x * x + y * y)};
+        double om[3];
+        for (int i = 0; i < 3; i++)
+            om[i] = R[3 * i] * yd[0] + R[3 * i + 1] * yd[1] + R[3 * i + 2] * yd[2];
+        // primal of the orientation, as integrateQuat computes it
+        const double t = sqrt(om[0] * om[0] + om[1] * om[1] + om[2] * om[2]);
+        double axis[3] = {1.0, 0.0, 0.0};
+        if (t > 0.0)
+            for (int i = 0; i < 3; i++)
+                axis[i] = om[i] / t;
+        double s, c;
+        sincos(0.5 * (t * dt), &s, &c);
+        const double d[4] = {c, s * axis[0], s * axis[1], s * axis[2]};
+        const double *qq = q + 3;
+        const double r[4] = {d[0] * qq[0] - d[1] * qq[1] - d[2] * qq[2] - d[3] * qq[3],
+                             d[0] * qq[1] + d[1] * qq[0] + d[2] * qq[3] - d[3] * qq[2],
+                             d[0] * qq[2] - d[1] * qq[3] + d[2] * qq[0] + d[3] * qq[1],
+                             d[0] * qq[3] + d[1] * qq[2] - d[2] * qq[1] + d[3] * qq[0]};
+        const double n = sqrt(r[0] * r[0] + r[1] * r[1] + r[2] * r[2] + r[3] * r[3]);
+        // out = r / n
+        const double *ob = q_out_bar + 3;
+        const double proj = (r[0] * ob[0] + r[1] * ob[1] + r[2] * ob[2] + r[3] * ob[3]) / (n * n);
+        double rb[4];
+        for (int i = 0; i < 4; i++)
+            rb[i] = (ob[i] - r[i] * proj) / n;
+        // r = d (x) quat
+        const double db[4] = {rb[0] * qq[0] + rb[1] * qq[1] + rb[2] * qq[2] + rb[3] * qq[3],
+                              -rb[0] * qq[1] + rb[1] * qq[0] - rb[2] * qq[3] + rb[3] * qq[2],
+                              -rb[0] * qq[2] + rb[1] * qq[3] + rb[2] * qq[0] - rb[3] * qq[1],
+                              -rb[0] * qq[3] - rb[1] * qq[2] + rb[2] * qq[1] + rb[3] * qq[0]};
+        double qb[4] = {rb[0] * d[0] + rb[1] * d[1] + rb[2] * d[2] + rb[3] * d[3],
+                        -rb[0] * d[1] + rb[1] * d[0] + rb[2] * d[3] - rb[3] * d[2],
+                        -rb[0] * d[2] - rb[1] * d[3] + rb[2] * d[0] + rb[3] * d[1],
+                        -rb[0] * d[3] + rb[1] * d[2] - rb[2] * d[1] + rb[3] * d[0]};
+        // d(omega)
+        const double a = 0.5 * dt, u = a * a * t * t;
+        double S, c2;
+        if (fabs(a) * t < 1e-2)
+        {
+            S = a * (1.0 - u / 6.0 * (1.0 - u / 20.0 * (1.0 - u / 42.0)));
+            c2 = -a * a * a / 3.0 * (1.0 - u / 10.0 * (1.0 - u / 28.0 * (1.0 - u / 54.0)));
+        }
+        else
+        {
+            S = s / t;
+            c2 = (a * c - S) / (t * t);
+        }
+        const double om_db = om[0] * db[1] + om[1] * db[2] + om[2] * db[3];
+        double omb[3], vb[3];
+        for (int i = 0; i < 3; i++)
+        {
+            omb[i] = -a * S * om[i] * db[0] + S * db[1 + i] + c2 * om[i] * om_db;
+            vb[i] = dt * q_out_bar[i]; // p' = p + dt R v_b
+            q_bar[i] = q_out_bar[i];
+        }
+        // om = R w_b, v = R v_b: R_bar = omb w_b^T + vb v_b^T, yd_bar += R^T [omb; vb]
+        double Rb[9];
+        for (int i = 0; i < 3; i++)
+            for (int j = 0; j < 3; j++)
+            {
+                Rb[3 * i + j] = omb[i] * yd[j] + vb[i] * yd[3 + j];
+                yd_bar[j] += R[3 * i + j] * omb[i];
+                yd_bar[3 + j] += R[3 * i + j] * vb[i];
+            }
+        qb[0] += 2 * (-Rb[1] * z + Rb[2] * y + Rb[3] * z - Rb[5] * x - Rb[6] * y + Rb[7] * x);
+        qb[1] += 2 * (Rb[1] * y + Rb[2] * z + Rb[3] * y - 2 * Rb[4] * x - Rb[5] * w + Rb[6] * z + Rb[7] * w - 2 * Rb[8] * x);
+        qb[2] += 2 * (-2 * Rb[0] * y + Rb[1] * x + Rb[2] * w + Rb[3] * x + Rb[5] * z - Rb[6] * w + Rb[7] * z - 2 * Rb[8] * y);
+        qb[3] += 2 * (-2 * Rb[0] * z - Rb[1] * w + Rb[2] * x + Rb[3] * w - 2 * Rb[4] * z + Rb[5] * y + Rb[6] * x + Rb[7] * y);
+        for (int i = 0; i < 4; i++)
+            q_bar[3 + i] = qb[i];
+    }
+
+    // Implicit cluster at its projected point q_span (projectImplicitPosition converged there), by the implicit
+    // function theorem: the new dependent coordinates are g(q_ind') with d g / d q_ind' = -K_dep^-1 K_ind, so
+    //   K_dep^T lambda = q_out_bar_dep,   q_ind_bar = q_out_bar_ind - K_ind^T lambda   (= G^T q_out_bar)
+    // and q_ind' = q_ind + dt yd_ind adds dt q_ind_bar to the cluster's velocities. The old dependent coordinates are
+    // only Newton's starting point: their q_bar is 0. C provides N, NC, ind(), dep() and
+    //   static void jacobian(const double *q, double *Kd, double *Ki)   (row-major per constraint).
+    template <typename C>
+    __device__ inline void implicitPositionVjp(const double *q_span, double dt, const double *q_out_bar, double *q_bar,
+                                               double *yd_bar)
+    {
+        constexpr int N = C::N, NC = C::NC, NI = N - NC;
+        double Kd[NC * NC], Ki[NC * NI], A[NC * NC], lambda[NC];
+        C::jacobian(q_span, Kd, Ki);
+        for (int i = 0; i < NC; i++)
+        {
+            for (int j = 0; j < NC; j++)
+                A[i * NC + j] = Kd[j * NC + i];
+            lambda[i] = q_out_bar[C::dep(i)];
+        }
+        if (!smallSolve<NC>(A, lambda))
+            for (int i = 0; i < NC; i++)
+                lambda[i] = nan("");
+        for (int k = 0; k < NI; k++)
+        {
+            double s = q_out_bar[C::ind(k)];
+            for (int i = 0; i < NC; i++)
+                s -= Ki[i * NI + k] * lambda[i];
+            q_bar[C::ind(k)] = s;
+            yd_bar[k] += dt * s;
+        }
+        for (int i = 0; i < NC; i++)
+            q_bar[C::dep(i)] = 0.0;
+    }
+
+    // One state of the reverse integration step. StepVjp::run(q, yd_new, dt, q_out_bar, q_bar, v_bar) is generated per
+    // model (compiler/compile.h emitIntegrateVjp): it re-runs the step cluster by cluster, Newton projections included,
+    // writes q_bar and adds the position part to v_bar. yd' = yd + dt ydd: yd_bar = v_bar, ydd_bar = dt v_bar.
+    template <typename StepVjp>
+    __device__ inline bool integrateVjpState(const double *q, const double *yd, const double *ydd, double dt,
+                                             const double *q_out_bar, const double *yd_out_bar, double *q_bar,
+                                             double *yd_bar, double *ydd_bar)
+    {
+        double ydn[StepVjp::NV];
+        for (int k = 0; k < StepVjp::NV; k++)
+        {
+            ydn[k] = yd[k] + dt * ydd[k];
+            yd_bar[k] = yd_out_bar[k];
+        }
+        const bool ok = StepVjp::run(q, ydn, dt, q_out_bar, q_bar, yd_bar);
+        for (int k = 0; k < StepVjp::NV; k++)
+            ydd_bar[k] = dt * yd_bar[k];
+        return ok;
+    }
+
+    template <typename StepVjp>
+    __global__ void __launch_bounds__(128)
+        grbda_integrate_vjp_kernel(const double *__restrict__ q, const double *__restrict__ yd,
+                                   const double *__restrict__ ydd, double dt, const double *__restrict__ q_out_bar,
+                                   const double *__restrict__ yd_out_bar, int64_t count, double *__restrict__ q_bar,
+                                   double *__restrict__ yd_bar, double *__restrict__ ydd_bar, int32_t *__restrict__ flags)
+    {
+        const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+        if (i >= count)
+            return;
+        constexpr int NQ = StepVjp::NQ, NV = StepVjp::NV;
+        double ql[NQ], ydl[NV], yddl[NV], qob[NQ], ydob[NV], qb[NQ], ydb[NV], yddb[NV];
+        for (int k = 0; k < NQ; k++)
+        {
+            ql[k] = q[i * NQ + k];
+            qob[k] = q_out_bar[i * NQ + k];
+        }
+        for (int k = 0; k < NV; k++)
+        {
+            ydl[k] = yd[i * NV + k];
+            yddl[k] = ydd[i * NV + k];
+            ydob[k] = yd_out_bar[i * NV + k];
+        }
+        const bool ok = integrateVjpState<StepVjp>(ql, ydl, yddl, dt, qob, ydob, qb, ydb, yddb);
+        for (int k = 0; k < NQ; k++)
+            q_bar[i * NQ + k] = qb[k];
+        for (int k = 0; k < NV; k++)
+        {
+            yd_bar[i * NV + k] = ydb[k];
+            ydd_bar[i * NV + k] = yddb[k];
+        }
+        if (flags)
+            flags[i] = ok ? 0 : 1;
+    }
+
     // Step::run advances one state (generated per model): semi-implicit Euler, yd' = yd + dt ydd, q' from yd'
     template <typename Step>
     __global__ void __launch_bounds__(128)

@@ -58,7 +58,8 @@ struct grbda_model
     mutable std::map<std::pair<cudaStream_t, int>, Scratch> scratch;
     // slot 0: tile flags of a launch; slot 1: intermediate generalized forces of the *_ext entry points;
     // slot 2: accelerations of grbda_cuda_step_f64; slot 3: packed inputs of the vector-Jacobian products;
-    // slot 4: the external-force contribution to q_bar of the *_ext_vjp entry points
+    // slot 4: the external-force contribution to q_bar of the *_ext_vjp entry points; slot 5: the integration part of
+    // grbda_cuda_step_vjp_f64 (q_bar, yd_bar) and its ydd_bar
     unsigned char *scratchFor(cudaStream_t stream, size_t bytes, int slot = 0) const
     {
         std::lock_guard<std::mutex> lock(scratch_mutex);
@@ -206,6 +207,14 @@ namespace
     }
     bool validEntry(int algo) { return algo >= 0 && algo < compiler::PROGRAM_COUNT && algo != compiler::PROGRAM_FD_LTL; }
 
+    // kernels compiled at run time for every model (programs that depend on caller-chosen sets, reverse mode)
+    void ensureExtJit(const grbda_model *m)
+    {
+        std::lock_guard<std::mutex> lock(m->jit_ext_mutex);
+        if (!m->jit_ext)
+            m->jit_ext.reset(new grbda_runtime::JitModel());
+    }
+
     grbda_status launchAlgo(const grbda_model *m, int algo, bool f32, const void *in0, const void *in1,
                             const void *in2, void *out0, void *out1, void *out2, int64_t batch, void *stream)
     {
@@ -227,9 +236,7 @@ namespace
         {
             if (grbda_runtime::jitMode() == 0)
                 return fail(GRBDA_ERR_NOT_COMPILED, "operational-space programs need run-time compilation (GRBDA_JIT=0)");
-            std::lock_guard<std::mutex> lock(m->jit_ext_mutex);
-            if (!m->jit_ext)
-                m->jit_ext.reset(new grbda_runtime::JitModel());
+            ensureExtJit(m);
         }
         const bool custom_forces = runtime_only || (m->jit_ext && !m->model.externalForceBodies().empty() &&
                                                     (algo == compiler::ALGO_GFA || algo == compiler::ALGO_GFS));
@@ -823,10 +830,20 @@ extern "C"
     // ---- kernel provenance / run-time compilation ------------------------------------------------------
     grbda_status grbda_cuda_model_prepare(const grbda_model *m, int algo, int f32)
     {
-        if (!m || !validEntry(algo))
+        if (!m || (algo != GRBDA_PROGRAM_INTEGRATE_VJP && !validEntry(algo)))
             return fail(GRBDA_ERR_INVALID_ARGUMENT, "bad arguments");
         if (m->device < 0 || !m->hasKernels())
             return fail(GRBDA_ERR_NO_DEVICE, "model was created without a CUDA device (host-only handle)");
+        if (algo == GRBDA_PROGRAM_INTEGRATE_VJP)
+        {
+            if (grbda_runtime::jitMode() == 0)
+                return fail(GRBDA_ERR_NOT_COMPILED, "the reverse integration step needs run-time compilation (GRBDA_JIT=0)");
+            ensureExtJit(m);
+            std::string err;
+            if (!grbda_runtime::jitPrepareIntegrateVjp(*m->jit_ext, m->model, m->device, err))
+                return fail(GRBDA_ERR_NOT_COMPILED, "reverse integration step: " + err);
+            return GRBDA_OK;
+        }
         if (algo >= compiler::ALGO_CONTACT_KIN)
             return fail(GRBDA_ERR_INVALID_ARGUMENT, "operational-space programs are compiled when first used");
         if (m->kernels)
@@ -876,14 +893,15 @@ extern "C"
     grbda_status grbda_cuda_jit_compile(const grbda_model *m, int algo, int f32, const char *source_path,
                                         const char *cubin_path)
     {
-        if (!m || (algo != -1 && !validEntry(algo)))
+        if (!m || (algo != -1 && algo != GRBDA_PROGRAM_INTEGRATE_VJP && !validEntry(algo)))
             return fail(GRBDA_ERR_INVALID_ARGUMENT, "bad arguments");
         return guarded([&]
                        {
             grbda_runtime::JitKernel k;
             std::vector<std::string> names, lowered;
-            const std::string src = algo < 0 ? grbda_runtime::jitGenerateSource(m->model, names)
-                                             : grbda_runtime::jitSource(m->model, algo, f32 != 0, k, names);
+            const std::string src = algo == -1 ? grbda_runtime::jitGenerateSource(m->model, names)
+                                    : algo == GRBDA_PROGRAM_INTEGRATE_VJP ? grbda_runtime::jitIntegrateVjpSource(m->model, names)
+                                                                          : grbda_runtime::jitSource(m->model, algo, f32 != 0, k, names);
             if (source_path)
             {
                 std::ofstream f(source_path);
@@ -1029,6 +1047,20 @@ namespace
         return launchAlgo(m, algo, false, q, yd, packed, q_bar, yd_bar, aux_bar, batch, stream);
     }
 
+    // y0 += x0, y1 += x1 (n0, n1 doubles) in one launch
+    grbda_status accumulate(double *y0, const double *x0, int64_t n0, double *y1, const double *x1, int64_t n1,
+                            cudaStream_t s)
+    {
+        const int64_t n = n0 + n1;
+        const int grid = (int)std::min<int64_t>((n + 255) / 256, 148 * 8);
+        grbda_kernels::accumulateKernel<<<grid, 256, 0, s>>>(y0, x0, n0, y1, x1, n1);
+        const cudaError_t e = cudaGetLastError();
+        if (e != cudaSuccess)
+            return cudaFail(e, "accumulateKernel");
+        g_launches++;
+        return GRBDA_OK;
+    }
+
     // The dynamics VJP with external forces, composed of the programs that exist (f_ext != NULL):
     //   inverse dynamics, tau = ID(q, yd, ydd) - J^T f: ALGO_ID_VJP with w, then ALGO_GFS_VJP(q, f, w);
     //   forward dynamics, ydd = FD(q, yd, tau'), tau' = tau + J^T f: ALGO_GFA -> tau' (scratch slot 1), ALGO_FD_VJP at
@@ -1066,14 +1098,7 @@ namespace
         else if ((st = launchVJP(m, compiler::ALGO_ID_VJP, q, yd, aux, w, q_bar, yd_bar, aux_bar, batch, stream)) != GRBDA_OK ||
                  (st = launchAlgo(m, compiler::ALGO_GFS_VJP, false, q, f_ext, w, q_gf, f_bar, nullptr, batch, stream)) != GRBDA_OK)
             return st;
-        const int64_t n = batch * nq;
-        const int grid = (int)std::min<int64_t>((n + 255) / 256, 148 * 8);
-        grbda_kernels::accumulateKernel<<<grid, 256, 0, s>>>(q_bar, q_gf, n);
-        const cudaError_t e = cudaGetLastError();
-        if (e != cudaSuccess)
-            return cudaFail(e, "accumulateKernel");
-        g_launches++;
-        return GRBDA_OK;
+        return accumulate(q_bar, q_gf, batch * nq, nullptr, nullptr, 0, s);
     }
 } // namespace
 
@@ -1183,6 +1208,66 @@ extern "C"
         if (st != GRBDA_OK)
             return st;
         return grbda_cuda_integrate_f64(m, q, yd, ydd, dt, q_out, yd_out, flags, batch, stream);
+    }
+
+    // ---- reverse mode of the integration step / simulation step -----------------------------------------------
+    grbda_status grbda_cuda_integrate_vjp_f64(const grbda_model *m, const double *q, const double *yd, const double *ydd,
+                                              double dt, const double *q_out_bar, const double *yd_out_bar,
+                                              double *q_bar, double *yd_bar, double *ydd_bar, int32_t *flags,
+                                              int64_t batch, void *stream)
+    {
+        grbda_status st = vjpCheck(m, batch);
+        if (st != GRBDA_OK || batch == 0)
+            return st;
+        if (!q || !yd || !ydd || !q_out_bar || !yd_out_bar)
+            return fail(GRBDA_ERR_INVALID_ARGUMENT, "null input pointer");
+        if (!q_bar || !yd_bar || !ydd_bar)
+            return fail(GRBDA_ERR_INVALID_ARGUMENT, "null output pointer");
+        DeviceScope scope(m->device);
+        if (scope.error != cudaSuccess)
+            return cudaFail(scope.error, "cudaSetDevice");
+        ensureExtJit(m);
+        std::string err;
+        if (!grbda_runtime::jitPrepareIntegrateVjp(*m->jit_ext, m->model, m->device, err))
+            return fail(GRBDA_ERR_NOT_COMPILED, "reverse integration step: " + err);
+        const grbda_runtime::StepVjpArgs a{q, yd, ydd, dt, q_out_bar, yd_out_bar, batch, q_bar, yd_bar, ydd_bar, flags,
+                                           (cudaStream_t)stream};
+        const cudaError_t e = grbda_runtime::jitLaunchIntegrateVjp(m->jit_ext->integrate_vjp, a);
+        if (e != cudaSuccess)
+            return cudaFail(e, "integrate vjp launch");
+        g_launches++;
+        return GRBDA_OK;
+    }
+
+    grbda_status grbda_cuda_step_vjp_f64(const grbda_model *m, const double *q, const double *yd, const double *tau,
+                                         const double *f_ext, double dt, const double *q_out_bar, const double *yd_out_bar,
+                                         double *q_bar, double *yd_bar, double *tau_bar, double *f_bar, int32_t *flags,
+                                         int64_t batch, void *stream)
+    {
+        grbda_status st = vjpCheck(m, batch);
+        if (st != GRBDA_OK || batch == 0)
+            return st;
+        if (!q || !yd || !tau || !q_out_bar || !yd_out_bar)
+            return fail(GRBDA_ERR_INVALID_ARGUMENT, "null input pointer");
+        if (!q_bar || !yd_bar || !tau_bar || (f_ext && !f_bar))
+            return fail(GRBDA_ERR_INVALID_ARGUMENT, "null output pointer");
+        DeviceScope scope(m->device);
+        if (scope.error != cudaSuccess)
+            return cudaFail(scope.error, "cudaSetDevice");
+        const cudaStream_t s = (cudaStream_t)stream;
+        const int64_t nq = m->model.getNumPositions(), nv = m->model.getNumDegreesOfFreedom();
+        double *ydd = (double *)m->scratchFor(s, (size_t)(batch * nv) * sizeof(double), 2);
+        double *bars = (double *)m->scratchFor(s, (size_t)(batch * (nq + 2 * nv)) * sizeof(double), 5);
+        if (!ydd || !bars)
+            return fail(GRBDA_ERR_CUDA, "cannot allocate the step scratch buffers: " + m->scratch_error);
+        double *q_bar_int = bars, *yd_bar_int = bars + batch * nq, *ydd_bar = yd_bar_int + batch * nv;
+        if ((st = grbda_cuda_forward_dynamics_ext_f64(m, q, yd, tau, f_ext, ydd, batch, stream)) != GRBDA_OK ||
+            (st = grbda_cuda_integrate_vjp_f64(m, q, yd, ydd, dt, q_out_bar, yd_out_bar, q_bar_int, yd_bar_int, ydd_bar,
+                                               flags, batch, stream)) != GRBDA_OK ||
+            (st = grbda_cuda_forward_dynamics_ext_vjp_f64(m, q, yd, tau, f_ext, ydd_bar, q_bar, yd_bar, tau_bar, f_bar,
+                                                          batch, stream)) != GRBDA_OK)
+            return st;
+        return accumulate(q_bar, q_bar_int, batch * nq, yd_bar, yd_bar_int, batch * nv, s);
     }
 
     // ---- host placement for the host-buffer path ------------------------------------------------------------

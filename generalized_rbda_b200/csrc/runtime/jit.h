@@ -46,6 +46,19 @@ namespace grbda_runtime
         std::mutex mutex;
         JitKernel algo[grbda::compiler::PROGRAM_COUNT][2]; // [entry point][0 f64, 1 f32] (slot 7 unused)
         JitKernel generate;
+        JitKernel integrate_vjp; // reverse integration step (jitIntegrateVjpSource)
+    };
+
+    // Arguments of grbda_integrate_vjp_kernel (kernels/stategen.cuh)
+    struct StepVjpArgs
+    {
+        const double *q, *yd, *ydd;
+        double dt;
+        const double *q_out_bar, *yd_out_bar;
+        int64_t count;
+        double *q_bar, *yd_bar, *ydd_bar;
+        int32_t *flags;
+        cudaStream_t stream;
     };
 
     // GRBDA_JIT: "0" never compile at run time, "force" ignore the ahead-of-time registry (tests), else: on a registry miss
@@ -59,15 +72,18 @@ namespace grbda_runtime
                     bool f32, std::string &error);
     bool jitPrepareGenerate(JitModel &jm, const grbda::ClusterTreeModel &model, uint64_t model_hash, int device,
                             std::string &error);
+    bool jitPrepareIntegrateVjp(JitModel &jm, const grbda::ClusterTreeModel &model, int device, std::string &error);
     cudaError_t jitLaunch(const JitKernel &k, bool f32, const LaunchArgs &a);
     cudaError_t jitLaunchGenerate(const JitKernel &k, const GenArgs &a);
     cudaError_t jitLaunchIntegrate(const JitKernel &k, const StepArgs &a); // k = JitModel::generate (second kernel of that module)
+    cudaError_t jitLaunchIntegrateVjp(const JitKernel &k, const StepVjpArgs &a); // k = JitModel::integrate_vjp
     void jitRelease(JitModel &jm);
 
     // The CUDA text handed to NVRTC for one entry point (tests compile it without a device).
     std::string jitSource(const grbda::ClusterTreeModel &model, int algo, bool f32, JitKernel &k,
                           std::vector<std::string> &name_expressions);
     std::string jitGenerateSource(const grbda::ClusterTreeModel &model, std::vector<std::string> &name_expressions);
+    std::string jitIntegrateVjpSource(const grbda::ClusterTreeModel &model, std::vector<std::string> &name_expressions);
     // NVRTC only (no device needed): cubin + lowered names. `log` receives the compiler log on failure.
     bool jitCompile(const std::string &source, const std::vector<std::string> &name_expressions,
                     std::vector<char> &cubin, std::vector<std::string> &lowered, std::string &log);

@@ -53,11 +53,16 @@ namespace grbda_kernels
         y[b] = m;
     }
 
-    // y[i] += x[i]: sums the two contributions to q_bar of the vector-Jacobian products with external forces
-    __global__ void __launch_bounds__(256) accumulateKernel(double *__restrict__ y, const double *__restrict__ x, int64_t n)
+    // y0[i] += x0[i] (i < n0), y1[i] += x1[i] (i < n1): sums the two contributions to q_bar of the vector-Jacobian
+    // products with external forces (n1 = 0), and to q_bar and yd_bar of the simulation step's
+    __global__ void __launch_bounds__(256) accumulateKernel(double *__restrict__ y0, const double *__restrict__ x0, int64_t n0,
+                                                            double *__restrict__ y1, const double *__restrict__ x1, int64_t n1)
     {
-        for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x)
-            y[i] += x[i];
+        for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n0 + n1; i += (int64_t)gridDim.x * blockDim.x)
+            if (i < n0)
+                y0[i] += x0[i];
+            else
+                y1[i - n0] += x1[i - n0];
     }
 
     // Dependent-free FMA streams: 8 independent accumulators per thread, `iters` rounds of 8 FMAs.

@@ -185,14 +185,18 @@ grbda_status grbda_cuda_kernel_counts(const grbda_model *m, int algo, int64_t *c
  * do (include/grbda/Dynamics/ClusterTreeModel.h:27-53). GRBDA_JIT=0 turns it off (create then fails
  * with GRBDA_ERR_NOT_COMPILED), GRBDA_JIT=force ignores the ahead-of-time kernels.
  * prepare: compile / load the kernels of one entry point now (algo 0 ID, 1 FD, 2 FK, 3 H, 4 phi,
- * 5 gfa, 6 gfs) instead of on first use, e.g. before capturing a CUDA graph. */
+ * 5 gfa, 6 gfs, GRBDA_PROGRAM_INTEGRATE_VJP) instead of on first use, e.g. before capturing a CUDA graph. */
 grbda_status grbda_cuda_model_prepare(const grbda_model *m, int algo, int f32);
+/* Program id of the reverse integration step (grbda_cuda_integrate_vjp_f64) for grbda_cuda_model_prepare and
+ * grbda_cuda_jit_compile; it is compiled at run time for every model, also for those built ahead of time. */
+#define GRBDA_PROGRAM_INTEGRATE_VJP (-2)
 /* info8 = {source (0 ahead of time, 1 run-time compiled), CTA size, CTAs per SM, dynamic shared
  * memory, program, flags (1 parked, 2 bulk-copy staged, 4 direct I/O, 8 loaded from the disk cache),
  * NVRTC milliseconds, ready}; fields 1-6 are reported for run-time compiled kernels only. */
 grbda_status grbda_cuda_kernel_info(const grbda_model *m, int algo, int f32, int64_t *info8);
 /* The run-time compiler without a device: writes the CUDA text of one entry point (algo -1: the
- * state generator) to source_path and / or the sm_100a cubin NVRTC makes of it to cubin_path. */
+ * state generator, GRBDA_PROGRAM_INTEGRATE_VJP: the reverse integration step) to source_path and / or the sm_100a
+ * cubin NVRTC makes of it to cubin_path. */
 grbda_status grbda_cuda_jit_compile(const grbda_model *m, int algo, int f32, const char *source_path,
                                     const char *cubin_path);
 
@@ -340,6 +344,45 @@ grbda_status grbda_cuda_integrate_f64(const grbda_model *m, const double *q, con
 grbda_status grbda_cuda_step_f64(const grbda_model *m, const double *q, const double *yd, const double *tau,
                                  const double *f_ext, double dt, double *q_out, double *yd_out, int32_t *flags,
                                  int64_t batch, void *stream);
+/* Reverse mode of the integration step, what the gradient of a loss over a rollout needs. For cotangents
+ * q_out_bar[batch][nq] and yd_out_bar[batch][nv] of (q_out, yd_out) = integrate(q, yd, ydd, dt):
+ *   v_bar = yd_out_bar + (d q_out / d yd')^T q_out_bar  (yd' = yd + dt ydd),  yd_bar = v_bar,  ydd_bar = dt v_bar,
+ *   q_bar = (d q_out / d q)^T q_out_bar,
+ * q_bar being the exact derivative of what the step computes for every stored position entry:
+ *   one-dof / explicit clusters: q_bar = q_out_bar, and dt q_out_bar enters v_bar;
+ *   quaternion base: the derivative of p + dt R(quat) v_body and of the renormalised product, R being the polynomial
+ *     of the raw stored entries (also off the unit sphere); finite and continuous at omega = 0 (Taylor series of the
+ *     rotation increment there);
+ *   implicit clusters: the converged projection differentiated by the implicit function theorem at the projected
+ *     point q': K_dep^T lambda = q_out_bar_dep, q_ind_bar = q_out_bar_ind - K_ind^T lambda (= G^T q_out_bar), and
+ *     dt q_ind_bar enters v_bar. The old dependent coordinates are only Newton's starting point: their q_bar is 0;
+ *   roll-pitch-yaw base: the step copies its positions, so q_bar = q_out_bar there, and the state is flagged.
+ * Each state's step is re-run (Newton included) by the kernel; there is no saved q_out to pass. flags (optional)
+ * receives the flags grbda_cuda_integrate_f64 writes; the values of a flagged state are the formula at the point
+ * where Newton stopped and are meaningless: mask them with the flags. One kernel launch, elementwise, compiled at
+ * run time (GRBDA_PROGRAM_INTEGRATE_VJP) for every model; GRBDA_JIT=0 gives GRBDA_ERR_NOT_COMPILED. batch = 0
+ * returns GRBDA_OK without launching anything. FP64 only. */
+grbda_status grbda_cuda_integrate_vjp_f64(const grbda_model *m, const double *q, const double *yd, const double *ydd,
+                                          double dt, const double *q_out_bar, const double *yd_out_bar,
+                                          double *q_bar, double *yd_bar, double *ydd_bar, int32_t *flags,
+                                          int64_t batch, void *stream);
+/* Reverse mode of grbda_cuda_step_f64 for the same cotangents: q_bar[batch][nq], yd_bar[batch][nv],
+ * tau_bar[batch][nv] and, when f_ext != NULL, f_bar[batch][nf][6] (f_ext = NULL: f_bar is not written and may be
+ * NULL). Launches, in order:
+ *   1. the forward dynamics ydd = FD(q, yd, tau [+ J^T f]) into the per-stream acceleration buffer, exactly as
+ *      grbda_cuda_step_f64 (the launches of grbda_cuda_forward_dynamics_ext_f64);
+ *   2. grbda_cuda_integrate_vjp_f64 at that ydd, its q_bar / yd_bar parts and ydd_bar to a per-stream scratch
+ *      buffer of the handle (one launch);
+ *   3. grbda_cuda_forward_dynamics_ext_vjp_f64 with that ydd_bar (its launches; without forces that is
+ *      grbda_cuda_forward_dynamics_vjp_f64);
+ *   4. one elementwise kernel that adds the integration parts to q_bar and yd_bar.
+ * q_bar: the integration part is exact as above; the dynamics part keeps the manifold convention of the
+ * forward-dynamics VJP. flags as for grbda_cuda_integrate_vjp_f64. The scratch buffers belong to the (handle,
+ * stream) pair, with the concurrency caveat of the VJP entry points above. FP64 only. */
+grbda_status grbda_cuda_step_vjp_f64(const grbda_model *m, const double *q, const double *yd, const double *tau,
+                                     const double *f_ext, double dt, const double *q_out_bar, const double *yd_out_bar,
+                                     double *q_bar, double *yd_bar, double *tau_bar, double *f_bar, int32_t *flags,
+                                     int64_t batch, void *stream);
 /* ydd = FD(q, yd, tau). Replaces setState + ClusterTreeModel::forwardDynamics(tau),
  * src/Dynamics/ClusterTreeDynamics.cpp:85-191. */
 grbda_status grbda_cuda_forward_dynamics_f64(const grbda_model *m, const double *q, const double *yd,

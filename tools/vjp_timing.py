@@ -10,8 +10,12 @@ TelloWithArms (default force bodies), Mini Cheetah and MIT humanoid with the con
 entry points, their VJPs, and for the contact kinematics the route contactJacobians + einsum (yd_bar = J_lin^T v_bar
 only) at the largest batch of 2^20, 2^19, ... whose J fits in half the free memory. No Jacobian entry point takes
 external forces, so the dynamics with forces have no Jacobian route.
+--step: the reverse integration and simulation steps, 2^20 states of the same four models: the integration kernel
+against the integration-VJP kernel, the step VJP against the forward-dynamics VJP alone, and the backward pass of a
+10-step grbda.autograd.step rollout (the loss weights the final q and yd) per step, timed alone after its forward pass.
 Usage: python tools/vjp_timing.py > profiles/r3_vjp.jsonl
-       python tools/vjp_timing.py --ext-contact > profiles/r4_ext_contact_vjp.jsonl"""
+       python tools/vjp_timing.py --ext-contact > profiles/r4_ext_contact_vjp.jsonl
+       python tools/vjp_timing.py --step > profiles/r5_step_vjp.jsonl"""
 import json
 import os
 import re
@@ -133,7 +137,62 @@ def ext_contact(gpu_name, power_limit):
         torch.cuda.empty_cache()
 
 
+def step_vjp(gpu_name, power_limit):
+    dt, steps = 1e-3, 10
+    for robot in ROBOTS:
+        m = grbda.ClusterTreeModel.from_robot(robot)
+        rec = {"model": robot, "nq": m.nq, "nv": m.nv, "gpu": gpu_name, "power_limit": power_limit}
+        q, yd, aux, _ = m.generateStates(128)
+        rec["integrate_vjp_first_call_s"] = first_call(
+            lambda: m.integrateVJP(q, yd, aux, dt, torch.rand_like(q), torch.rand_like(yd)))
+        tool = shutil.which("cuobjdump") or "/usr/local/cuda/bin/cuobjdump"
+        if os.path.exists(tool):
+            path = os.path.join(WORK.name, "integrate_vjp_%s.cubin" % robot)
+            m.jit_compile(grbda.PROGRAM_INTEGRATE_VJP, False, None, path)
+            usage = re.findall(r"REG:(\d+) STACK:(\d+)", subprocess.run([tool, "-res-usage", path], capture_output=True,
+                                                                         text=True).stdout)
+            if usage:
+                rec["integrate_vjp_registers"] = max(int(r) for r, _ in usage)
+                rec["integrate_vjp_stack_bytes"] = max(int(st) for _, st in usage)
+        B = 1 << 20
+        rec["states"] = B
+        q, yd, aux, _ = m.generateStates(B)
+        qob, ydob = torch.rand_like(q) * 2 - 1, torch.rand_like(yd) * 2 - 1
+        rec["flagged_states"] = int(m.integrate(q, yd, aux, dt)[2].sum())
+        rec["integrate_ms"] = round(timeit(lambda: m.integrate(q, yd, aux, dt)), 4)
+        rec["integrate_vjp_ms"] = round(timeit(lambda: m.integrateVJP(q, yd, aux, dt, qob, ydob)), 4)
+        rec["step_ms"] = round(timeit(lambda: m.step(q, yd, aux, dt)), 4)
+        rec["fd_vjp_ms"] = round(timeit(lambda: m.forwardDynamicsVJP(q, yd, aux, ydob)), 4)
+        rec["step_vjp_ms"] = round(timeit(lambda: m.stepVJP(q, yd, aux, dt, qob, ydob)), 4)
+        # rollout: forward (not timed), then the backward alone between two events
+        times = []
+        for rep in range(4):
+            tau = aux.clone().requires_grad_(True)
+            qt, ydt = q, yd
+            for _ in range(steps):
+                qt, ydt, _ = grbda.autograd.step(m, qt, ydt, tau, dt)
+            loss = (qt * qob).sum() + (ydt * ydob).sum()
+            a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            torch.cuda.synchronize()
+            a.record()
+            loss.backward()
+            b.record()
+            torch.cuda.synchronize()
+            if rep:
+                times.append(a.elapsed_time(b) / steps)
+            del tau, qt, ydt, loss
+        rec["rollout_backward_ms_per_step"] = round(sorted(times)[len(times) // 2], 4)
+        rec["rollout_steps"] = steps
+        print(json.dumps(rec), flush=True)
+        del q, yd, aux, qob, ydob
+        torch.cuda.empty_cache()
+
+
 gpu_name, power_limit = card()
+if "--step" in sys.argv:
+    step_vjp(gpu_name, power_limit)
+    WORK.cleanup()
+    sys.exit(0)
 if "--ext-contact" in sys.argv:
     ext_contact(gpu_name, power_limit)
     WORK.cleanup()
