@@ -34,6 +34,7 @@ ALGO_CONTACT_KIN, ALGO_CONTACT_JAC, ALGO_TEST_FORCE, ALGO_OSIM = 8, 9, 10, 11  #
 ALGO_ID_DERIV, ALGO_FD_DERIV = 12, 13  # derivatives of the dynamics
 ALGO_ID_VJP, ALGO_FD_VJP = 14, 15  # vector-Jacobian products of the dynamics (reverse mode)
 ALGO_GFA_VJP, ALGO_GFS_VJP, ALGO_CONTACT_KIN_VJP = 16, 17, 18  # ... of the external-force programs, contact kinematics
+ALGO_CONTACT_FD, ALGO_CONTACT_IMPULSE = 19, 20  # rigid point contacts: constrained forward dynamics, impulses
 PROGRAM_FD_LTL = 7  # dump_program only: forward dynamics as CRBA + bias + sparse L^T D L (kernel variant "ltl")
 PROGRAM_INTEGRATE_VJP = -2  # prepare / jit_compile: the reverse integration step (GRBDA_PROGRAM_INTEGRATE_VJP)
 
@@ -86,6 +87,8 @@ _lib.grbda_cuda_forward_dynamics_vjp_f64.argtypes = [_vp, _vp, _vp, _vp, _vp, _v
 _lib.grbda_cuda_inverse_dynamics_ext_vjp_f64.argtypes = [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _vp]
 _lib.grbda_cuda_forward_dynamics_ext_vjp_f64.argtypes = [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _vp]
 _lib.grbda_cuda_contact_kinematics_vjp_f64.argtypes = [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _vp]
+_lib.grbda_cuda_contact_forward_dynamics_f64.argtypes = [_vp, _vp, _vp, _vp, _vp, C.c_double, _vp, _vp, _i64, _vp]
+_lib.grbda_cuda_contact_impulse_f64.argtypes = [_vp, _vp, _vp, _vp, C.c_double, C.c_double, _vp, _vp, _i64, _vp]
 _lib.grbda_cuda_integrate_f64.argtypes = [_vp, _vp, _vp, _vp, C.c_double, _vp, _vp, _vp, _i64, _vp]
 _lib.grbda_cuda_step_f64.argtypes = [_vp, _vp, _vp, _vp, _vp, C.c_double, _vp, _vp, _vp, _i64, _vp]
 _lib.grbda_cuda_integrate_vjp_f64.argtypes = [_vp, _vp, _vp, _vp, C.c_double, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _vp]
@@ -115,7 +118,7 @@ EXPORTED_SYMBOLS = [
     "grbda_cuda_inverse_dynamics_derivatives_f64", "grbda_cuda_forward_dynamics_derivatives_f64",
     "grbda_cuda_inverse_dynamics_vjp_f64", "grbda_cuda_forward_dynamics_vjp_f64",
     "grbda_cuda_inverse_dynamics_ext_vjp_f64", "grbda_cuda_forward_dynamics_ext_vjp_f64",
-    "grbda_cuda_contact_kinematics_vjp_f64",
+    "grbda_cuda_contact_kinematics_vjp_f64", "grbda_cuda_contact_forward_dynamics_f64", "grbda_cuda_contact_impulse_f64",
     "grbda_cuda_inverse_dynamics_f64", "grbda_cuda_inverse_dynamics_f32",
     "grbda_cuda_forward_dynamics_f64", "grbda_cuda_forward_dynamics_f32",
     "grbda_cuda_mass_matrix_f64", "grbda_cuda_mass_matrix_f32",
@@ -565,6 +568,48 @@ class ClusterTreeModel:
         L = torch.empty((q.shape[0], n, n), dtype=torch.float64, device=q.device)
         _check(_lib.grbda_cuda_inverse_osim_f64(self._h, _ptr(q), _ptr(L), q.shape[0], _stream()))
         return L
+
+    def _active(self, active, B):
+        import torch
+        if active is None:
+            return None
+        if not active.is_cuda or active.dtype not in (torch.bool, torch.uint8):
+            raise ValueError("active must be a bool or uint8 CUDA tensor")
+        if active.dim() != 2 or tuple(active.shape) != (B, self.ncp) or not active.is_contiguous():
+            raise ValueError("expected a contiguous [batch, %d] mask, got %s" % (self.ncp, tuple(active.shape)))
+        if self.device is not None and active.device.index != self.device:
+            raise ValueError("tensor lives on cuda:%d but the model was created on cuda:%d" % (active.device.index, self.device))
+        return active
+
+    def contactForwardDynamics(self, q, yd, tau, active=None, damping=0.0):
+        """(ydd[batch, nv], lam[batch, n_cp, 3]): forward dynamics with the active contact points held by rigid
+        bilateral contacts, lam the world-frame contact forces (include/grbda_cuda.h). active[batch, n_cp] (bool or
+        uint8; None: all active) selects the contacts per state; damping >= 0 regularises A (needed when the active
+        points are redundant, e.g. two points on one foot)."""
+        import torch
+        q = self._prep(q, self.nq, torch.float64)
+        yd, tau = self._prep(yd, self.nv, torch.float64), self._prep(tau, self.nv, torch.float64)
+        B = q.shape[0]
+        a = self._active(active, B)
+        ydd = torch.empty_like(tau)
+        lam = torch.empty((B, self.ncp, 3), dtype=torch.float64, device=q.device)
+        _check(_lib.grbda_cuda_contact_forward_dynamics_f64(self._h, _ptr(q), _ptr(yd), _ptr(tau), _ptr(a), float(damping),
+                                                            _ptr(ydd), _ptr(lam), B, _stream()))
+        return ydd, lam
+
+    def contactImpulse(self, q, yd, active=None, restitution=0.0, damping=0.0):
+        """(yd_plus[batch, nv], impulse[batch, n_cp, 3]): the velocity after an impact of the active contact points
+        and the world-frame impulses, J_a yd_plus = -restitution J_a yd - damping impulse_a (include/grbda_cuda.h)."""
+        import torch
+        q = self._prep(q, self.nq, torch.float64)
+        yd = self._prep(yd, self.nv, torch.float64)
+        B = q.shape[0]
+        a = self._active(active, B)
+        yd_plus = torch.empty_like(yd)
+        imp = torch.empty((B, self.ncp, 3), dtype=torch.float64, device=q.device)
+        _check(_lib.grbda_cuda_contact_impulse_f64(self._h, _ptr(q), _ptr(yd), _ptr(a), float(restitution), float(damping),
+                                                   _ptr(yd_plus), _ptr(imp), B, _stream()))
+        return yd_plus, imp
 
     def inverseDynamicsDerivatives(self, q, yd, ydd):
         """(dtau_dq, dtau_dyd), each [batch, nv, nv], [b, i, j] = d tau_i / d x_j; dq is the tangent-space

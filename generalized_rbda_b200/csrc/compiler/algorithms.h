@@ -1811,6 +1811,100 @@ namespace grbda
                 return out;
             }
 
+            // Rigid point contacts (include/grbda_cuda.h): J (m = 3 n_cp rows) stacks the linear world rows of
+            // contactJacobianWorld, s the per-contact activity mask (S = diag(s (x) 1_3)), eps the damping:
+            //   A = S (J Y) S + (I - S) + eps I,   Y = H^-1 J^T (m solves, one factorisation),
+            //   dynamics (impulse = false): in2 = [tau; s; eps], ydd0 = H^-1 (tau - C), b = -S (J ydd0 + c),
+            //                               out = ydd0 + Y lambda,   lambda = A^-1 b,
+            //   impulse  (impulse = true):  in2 = [s; e; eps], b = -(1 + e) S J yd, out = yd + Y lambda.
+            // c = Jdot yd is the classical world acceleration of every contact point at ydd = 0 without gravity. J and
+            // c use the true poses of contactSetup; ydd0, H and the factor the dynamics' own reductions. A masked row
+            // and column of A and the masked entries of b are exact zeros, so its lambda is exactly zero after the
+            // unrolled LDL^T (no pivoting: with eps = 0 the active rows of J must be linearly independent).
+            void contactDynamics(bool impulse, std::vector<Sym> &out, std::vector<Sym> &lambda)
+            {
+                const int nv = m_.getNumDegreesOfFreedom(), ncp = (int)m_.contactPoints().size(), m = 3 * ncp;
+                const int s0 = impulse ? 0 : nv; // mask position in input array 2
+                std::vector<std::vector<Sym>> J;
+                std::vector<Sym> c;
+                {
+                    std::vector<Xf> Xa;
+                    contactSetup(!impulse, Xa);
+                    std::vector<SV> a(m_.getNumBodies()); // body accelerations at ydd = 0, zero gravity (inverseDynamics)
+                    if (!impulse)
+                        for (const ClusterTreeNode &cl : m_.clusters())
+                        {
+                            const ClusterDesc &d = cl.joint_;
+                            const bool is_free = d.type == ClusterType::FreeQuaternion || d.type == ClusterType::FreeRollPitchYaw;
+                            for (int i = 0; i < d.num_bodies; i++)
+                            {
+                                const int bi = cl.first_body_ + i, p = m_.bodies()[bi].parent_index_;
+                                SV ai = p >= 0 ? bk_[bi].Xl.applyMotion(a[p]) : SV();
+                                if (!is_free)
+                                {
+                                    const int axis = (int)d.axes[i];
+                                    SV sq;
+                                    sq[axis] = bk_[bi].qd;
+                                    ai[axis] = ai[axis] + ck_[cl.index_].g[i];
+                                    ai = ai + motionCross(bk_[bi].v, sq);
+                                }
+                                a[bi] = ai;
+                            }
+                        }
+                    for (const ContactPoint &cp : m_.contactPoints())
+                    {
+                        const auto Jw = contactJacobianWorld(cp, Xa);
+                        for (int r = 0; r < 3; r++)
+                            J.push_back(Jw[3 + r]);
+                        if (impulse)
+                            continue;
+                        const SV &v = bk_[cp.body_index_].v, &ad = a[cp.body_index_];
+                        const V3 d = constV3(cp.local_offset_), w = v.ang();
+                        const V3 acc = ad.lin() + cross(w, v.lin()) + cross(ad.ang(), d) + cross(w, cross(w, d));
+                        const V3 cw = mulT(Xa[cp.body_index_].E, acc);
+                        for (int r = 0; r < 3; r++)
+                            c.push_back(cw[r]);
+                    }
+                }
+                std::vector<Sym> base(nv), s(m), b(m);
+                if (impulse)
+                    for (int k = 0; k < nv; k++)
+                        base[k] = Sym::input(IN_YD, k);
+                else
+                    base = forwardDynamicsLTL();
+                const Sym eps = Sym::input(IN_AUX, s0 + ncp + (impulse ? 1 : 0));
+                const Sym gain = impulse ? Sym(1.0) + Sym::input(IN_AUX, s0 + ncp) : Sym(1.0);
+                for (int i = 0; i < m; i++)
+                {
+                    s[i] = Sym::input(IN_AUX, s0 + i / 3);
+                    Sym jx(0.0);
+                    for (int k = 0; k < nv; k++)
+                        jx = jx + J[i][k] * base[k];
+                    b[i] = impulse ? -(gain * (s[i] * jx)) : -(s[i] * (jx + c[i]));
+                }
+                std::vector<std::vector<Sym>> Y(m);
+                for (int i = 0; i < m; i++)
+                    Y[i] = solveMassMatrix(J[i]);
+                std::vector<Sym> A(m * m, Sym(0.0)); // lower triangle: all LDLT reads
+                for (int i = 0; i < m; i++)
+                    for (int j = 0; j <= i; j++)
+                    {
+                        Sym jy(0.0);
+                        for (int k = 0; k < nv; k++)
+                            jy = jy + J[i][k] * Y[j][k];
+                        A[i * m + j] = s[i] * (s[j] * jy);
+                        if (i == j)
+                            A[i * m + j] = A[i * m + j] + (Sym(1.0) - s[i]) + eps;
+                    }
+                LDLT f;
+                f.factor(A, m);
+                lambda = f.solve(b);
+                out = base;
+                for (int k = 0; k < nv; k++)
+                    for (int i = 0; i < m; i++)
+                        out[k] = out[k] + Y[i][k] * lambda[i];
+            }
+
             const std::vector<BodyKin> &bodyKinematics() const { return bk_; }
             const std::vector<ClusterKin> &clusterKinematics() const { return ck_; }
 

@@ -42,7 +42,10 @@ namespace grbda
             ALGO_GFA_VJP = 16,     // in: q, f_ext [6 nf], w [nv]   out: q_bar [nq], f_bar = J w [6 nf]
             ALGO_GFS_VJP = 17,     // in: q, f_ext [6 nf], w [nv]   out: q_bar [nq], f_bar = -J w [6 nf]
             ALGO_CONTACT_KIN_VJP = 18, // in: q, yd, [p_bar; v_bar] [6 n_cp]   out: q_bar [nq], yd_bar = J_lin^T v_bar [nv]
-            PROGRAM_COUNT = 19
+            // rigid point contacts (ModelCompiler::contactDynamics): s = activity mask [n_cp], eps = damping
+            ALGO_CONTACT_FD = 19,      // in: q, yd, [tau; s; eps]   out: ydd [nv], lambda [3 n_cp] (world forces)
+            ALGO_CONTACT_IMPULSE = 20, // in: q, yd, [s; e; eps]     out: yd_plus [nv], impulse [3 n_cp]
+            PROGRAM_COUNT = 21
         };
         // registry slot a program belongs to
         inline int algoOfProgram(int program) { return program == PROGRAM_FD_LTL ? ALGO_FD : program; }
@@ -50,7 +53,7 @@ namespace grbda
         {
             static const char *names[] = {"id", "fd", "fk", "h", "phi", "gfa", "gfs", "fd_ltl", "contact_kin", "contact_jac",
                                           "test_force", "osim", "id_deriv", "fd_deriv", "id_vjp", "fd_vjp", "gfa_vjp", "gfs_vjp",
-                                          "contact_kin_vjp"};
+                                          "contact_kin_vjp", "contact_fd", "contact_impulse"};
             return names[a];
         }
 
@@ -134,6 +137,15 @@ namespace grbda
             case ALGO_CONTACT_KIN_VJP:
                 n_in[1] = nv, n_in[2] = 6 * (int)model.contactPoints().size(), n_out[0] = nq, n_out[1] = nv;
                 break;
+            case ALGO_CONTACT_FD:
+            case ALGO_CONTACT_IMPULSE:
+            {
+                // no contact points: no program (n_out[0] = 0 marks an entry point that does not exist)
+                const int ncp = (int)model.contactPoints().size();
+                n_in[1] = nv, n_in[2] = (program == ALGO_CONTACT_FD ? nv + ncp + 1 : ncp + 2);
+                n_out[0] = ncp ? nv : 0, n_out[1] = 3 * ncp;
+                break;
+            }
             default:
                 throw std::runtime_error("algoSizes: unknown program");
             }
@@ -269,6 +281,18 @@ namespace grbda
                 std::vector<sym::Sym> q_bar, yd_bar;
                 mc.contactKinematicsVJP(q_bar, yd_bar);
                 p.outputs = {q_bar, yd_bar};
+                break;
+            }
+            case ALGO_CONTACT_FD:
+            case ALGO_CONTACT_IMPULSE:
+            {
+                const int ncp = (int)model.contactPoints().size();
+                if (ncp == 0)
+                    throw std::runtime_error("contact dynamics: the model has no contact points");
+                p.n_in[0] = nq, p.n_in[1] = nv, p.n_in[2] = algo == ALGO_CONTACT_FD ? nv + ncp + 1 : ncp + 2;
+                std::vector<sym::Sym> y, lambda;
+                mc.contactDynamics(algo == ALGO_CONTACT_IMPULSE, y, lambda);
+                p.outputs = {y, lambda};
                 break;
             }
             default:

@@ -4,6 +4,7 @@
 // there is deliberately no CPU evaluation path.
 #include <algorithm>
 #include <atomic>
+#include <cmath>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -844,6 +845,18 @@ extern "C"
                 return fail(GRBDA_ERR_NOT_COMPILED, "reverse integration step: " + err);
             return GRBDA_OK;
         }
+        if (algo == compiler::ALGO_CONTACT_FD || algo == compiler::ALGO_CONTACT_IMPULSE)
+        {
+            if (grbda_runtime::jitMode() == 0)
+                return fail(GRBDA_ERR_NOT_COMPILED, "rigid-contact programs need run-time compilation (GRBDA_JIT=0)");
+            if (f32 || m->model.contactPoints().empty())
+                return fail(GRBDA_ERR_INVALID_ARGUMENT, "rigid-contact programs: FP64 and a contact set only");
+            ensureExtJit(m);
+            std::string err;
+            if (!grbda_runtime::jitPrepare(*m->jit_ext, m->model, m->hash, m->device, algo, false, err))
+                return fail(GRBDA_ERR_NOT_COMPILED, err);
+            return GRBDA_OK;
+        }
         if (algo >= compiler::ALGO_CONTACT_KIN)
             return fail(GRBDA_ERR_INVALID_ARGUMENT, "operational-space programs are compiled when first used");
         if (m->kernels)
@@ -946,7 +959,8 @@ extern "C"
             std::lock_guard<std::mutex> lock(m->jit_ext_mutex);
             if (m->jit_ext)
                 for (int a : {compiler::ALGO_CONTACT_KIN, compiler::ALGO_CONTACT_JAC, compiler::ALGO_TEST_FORCE,
-                              compiler::ALGO_OSIM, compiler::ALGO_CONTACT_KIN_VJP})
+                              compiler::ALGO_OSIM, compiler::ALGO_CONTACT_KIN_VJP, compiler::ALGO_CONTACT_FD,
+                              compiler::ALGO_CONTACT_IMPULSE})
                     for (int p = 0; p < 2; p++)
                     {
                         if (m->jit_ext->algo[a][p].library)
@@ -1100,6 +1114,53 @@ namespace
             return st;
         return accumulate(q_bar, q_gf, batch * nq, nullptr, nullptr, 0, s);
     }
+
+    // The rigid-contact programs (include/grbda_cuda.h): packContactRowsKernel writes input array 2 into scratch slot 3
+    // (the packed inputs of the VJPs), then the program runs, both on the caller's stream
+    grbda_status launchContact(const grbda_model *m, int algo, const double *q, const double *yd, const double *tau,
+                               const uint8_t *active, double restitution, double damping, double *y_out, double *lambda,
+                               int64_t batch, void *stream)
+    {
+        if (!m)
+            return fail(GRBDA_ERR_INVALID_ARGUMENT, "null model");
+        if (m->model.contactPoints().empty())
+            return fail(GRBDA_ERR_INVALID_ARGUMENT, "the model has no contact points (grbda_cuda_set_contact_points)");
+        if (!std::isfinite(damping) || damping < 0.0)
+            return fail(GRBDA_ERR_INVALID_ARGUMENT, "the damping must be finite and >= 0");
+        if (!(restitution >= 0.0 && restitution <= 1.0))
+            return fail(GRBDA_ERR_INVALID_ARGUMENT, "the restitution must lie in [0, 1]");
+        if (m->device < 0 || !m->hasKernels())
+            return fail(GRBDA_ERR_NO_DEVICE, "model was created without a CUDA device (host-only handle)");
+        if (batch < 0)
+            return fail(GRBDA_ERR_INVALID_ARGUMENT, "negative batch");
+        if (grbda_runtime::jitMode() == 0)
+            return fail(GRBDA_ERR_NOT_COMPILED, "rigid-contact programs need run-time compilation (GRBDA_JIT=0)");
+        if (batch == 0)
+            return GRBDA_OK;
+        const bool impulse = algo == compiler::ALGO_CONTACT_IMPULSE;
+        if (!q || !yd || (!impulse && !tau))
+            return fail(GRBDA_ERR_INVALID_ARGUMENT, "null input pointer");
+        if (!y_out || !lambda)
+            return fail(GRBDA_ERR_INVALID_ARGUMENT, "null output pointer");
+        DeviceScope scope(m->device);
+        if (scope.error != cudaSuccess)
+            return cudaFail(scope.error, "cudaSetDevice");
+        const cudaStream_t s = (cudaStream_t)stream;
+        const int ncp = (int)m->model.contactPoints().size(), nt = impulse ? 0 : m->model.getNumDegreesOfFreedom();
+        const int ns = impulse ? 2 : 1;
+        const int64_t n = batch * (nt + ncp + ns);
+        double *packed = (double *)m->scratchFor(s, (size_t)n * sizeof(double), 3);
+        if (!packed)
+            return fail(GRBDA_ERR_CUDA, "cannot allocate the packed input buffer: " + m->scratch_error);
+        const int grid = (int)std::min<int64_t>((n + 255) / 256, 148 * 8);
+        grbda_kernels::packContactRowsKernel<<<grid, 256, 0, s>>>(packed, tau, nt, active, ncp, impulse ? restitution : damping,
+                                                                 damping, ns, batch);
+        const cudaError_t e = cudaGetLastError();
+        if (e != cudaSuccess)
+            return cudaFail(e, "packContactRowsKernel");
+        g_launches++;
+        return launchAlgo(m, algo, false, q, yd, packed, y_out, lambda, nullptr, batch, stream);
+    }
 } // namespace
 
 extern "C"
@@ -1153,6 +1214,19 @@ extern "C"
         if ((st = packRows(m, p_bar, n, v_bar, n, batch, (cudaStream_t)stream, packed)) != GRBDA_OK)
             return st;
         return launchAlgo(m, compiler::ALGO_CONTACT_KIN_VJP, false, q, yd, packed, q_bar, yd_bar, nullptr, batch, stream);
+    }
+    grbda_status grbda_cuda_contact_forward_dynamics_f64(const grbda_model *m, const double *q, const double *yd,
+                                                         const double *tau, const uint8_t *active, double damping,
+                                                         double *ydd, double *lambda, int64_t batch, void *stream)
+    {
+        return launchContact(m, compiler::ALGO_CONTACT_FD, q, yd, tau, active, 0.0, damping, ydd, lambda, batch, stream);
+    }
+    grbda_status grbda_cuda_contact_impulse_f64(const grbda_model *m, const double *q, const double *yd,
+                                                const uint8_t *active, double restitution, double damping,
+                                                double *yd_plus, double *impulse, int64_t batch, void *stream)
+    {
+        return launchContact(m, compiler::ALGO_CONTACT_IMPULSE, q, yd, nullptr, active, restitution, damping, yd_plus,
+                             impulse, batch, stream);
     }
     grbda_status grbda_cuda_inverse_osim_f64(const grbda_model *m, const double *q, double *lambda_inv, int64_t batch,
                                              void *stream)

@@ -1,5 +1,5 @@
 // Small hand-written support kernels: checksum, row-wise max |x| (constraint violation), elementwise
-// accumulation, FMA peak micro-benchmark (the FP64 / FP32 roofline denominators are measured, not assumed).
+// accumulation, packing of the rigid-contact inputs, FMA peak micro-benchmark (the FP64 / FP32 roofline denominators are measured, not assumed).
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -63,6 +63,29 @@ namespace grbda_kernels
                 y0[i] += x0[i];
             else
                 y1[i - n0] += x1[i - n0];
+    }
+
+    // Input array 2 of the rigid-contact programs, row b = [tau[b] (nt values); s (ncp); x0 (, x1)] with s_k = 1.0 where
+    // active[b][k] != 0, 0.0 elsewhere, all 1.0 without a mask (active = NULL); ns = 1 or 2 scalars broadcast to every
+    // row: [tau; s; eps] (nt = nv, ns = 1) for the contact dynamics, [s; e; eps] (nt = 0, ns = 2) for the impulse
+    __global__ void __launch_bounds__(256) packContactRowsKernel(double *__restrict__ packed, const double *__restrict__ tau,
+                                                                 int nt, const uint8_t *__restrict__ active, int ncp,
+                                                                 double x0, double x1, int ns, int64_t batch)
+    {
+        const int row = nt + ncp + ns;
+        for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < batch * row; i += (int64_t)gridDim.x * blockDim.x)
+        {
+            const int64_t b = i / row;
+            const int k = (int)(i - b * row);
+            double v;
+            if (k < nt)
+                v = tau[b * nt + k];
+            else if (k < nt + ncp)
+                v = !active || active[b * ncp + (k - nt)] ? 1.0 : 0.0;
+            else
+                v = k == nt + ncp ? x0 : x1;
+            packed[i] = v;
+        }
     }
 
     // Dependent-free FMA streams: 8 independent accumulators per thread, `iters` rounds of 8 FMAs.

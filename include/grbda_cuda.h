@@ -185,7 +185,8 @@ grbda_status grbda_cuda_kernel_counts(const grbda_model *m, int algo, int64_t *c
  * do (include/grbda/Dynamics/ClusterTreeModel.h:27-53). GRBDA_JIT=0 turns it off (create then fails
  * with GRBDA_ERR_NOT_COMPILED), GRBDA_JIT=force ignores the ahead-of-time kernels.
  * prepare: compile / load the kernels of one entry point now (algo 0 ID, 1 FD, 2 FK, 3 H, 4 phi,
- * 5 gfa, 6 gfs, GRBDA_PROGRAM_INTEGRATE_VJP) instead of on first use, e.g. before capturing a CUDA graph. */
+ * 5 gfa, 6 gfs, 19 contact forward dynamics, 20 contact impulse (FP64, for the current contact set),
+ * GRBDA_PROGRAM_INTEGRATE_VJP) instead of on first use, e.g. before capturing a CUDA graph. */
 grbda_status grbda_cuda_model_prepare(const grbda_model *m, int algo, int f32);
 /* Program id of the reverse integration step (grbda_cuda_integrate_vjp_f64) for grbda_cuda_model_prepare and
  * grbda_cuda_jit_compile; it is compiled at run time for every model, also for those built ahead of time. */
@@ -254,6 +255,44 @@ grbda_status grbda_cuda_apply_test_force_f64(const grbda_model *m, const double 
  * (the extended force propagator algorithm), src/Dynamics/ClusterTreeDynamics.cpp:292-435. */
 grbda_status grbda_cuda_inverse_osim_f64(const grbda_model *m, const double *q, double *lambda_inv, int64_t batch,
                                          void *stream);
+/* ---- rigid point contacts: contact-constrained forward dynamics and contact impulses --------------------------- */
+/* The contact points are those of grbda_cuda_set_contact_points, n_c of them, m = 3 n_c. J (m x nv) stacks the LINEAR
+ * rows (3..5) of each contact's world-frame Jacobian, as applyTestForce uses them. active[batch][n_c] is a per-state
+ * activity mask s (nonzero = active; active = NULL: all active), S = diag(s (x) 1_3); damping eps >= 0 is one value per
+ * call. c = Jdot yd is the classical world-frame acceleration of every contact point at ydd = 0, WITHOUT gravity: with
+ * (w, v_o) the spatial velocity and (wdot, a_o) the spatial acceleration of the body (body coordinates, ydd = 0, zero
+ * gravity), d the offset and E the body's rotation (world -> body),
+ *   c_k = E^T (a_o + w x v_o + wdot x d + w x (w x d)).
+ * Both entry points share
+ *   Y = H^-1 J^T (m solves with one factorisation),   A = S (J Y) S + (I - S) + eps I,
+ * and solve A x = b with an unrolled LDL^T of the m x m matrix.
+ * Contact-constrained forward dynamics: tau[batch][nv] in, ydd[batch][nv] and lambda[batch][n_c][3] out:
+ *   ydd0 = H^-1 (tau - C) (what grbda_cuda_forward_dynamics_f64 returns),  b = -S (J ydd0 + c),
+ *   lambda = A^-1 b,  ydd = ydd0 + Y lambda.
+ * lambda is the world-frame force applied to the robot at each contact point. The result satisfies H ydd + C =
+ * tau + J^T lambda; J_a ydd + c_a = -eps lambda_a for the active contacts; lambda = 0 exactly for the inactive ones
+ * (their rows and columns of A and their entries of b are exact zeros, which the factorisation keeps while the values
+ * are finite).
+ * Contact impulse: yd[batch][nv] is the velocity before the impact, yd_plus[batch][nv] the velocity after it and
+ * impulse[batch][n_c][3] the world-frame impulse at each contact point; restitution e in [0, 1]:
+ *   b = -(1 + e) S J yd,  impulse = A^-1 b,  yd_plus = yd + Y impulse,
+ * so that J_a yd_plus = -e J_a yd - eps impulse_a and impulse = 0 for the inactive contacts.
+ * The factorisation has no pivoting (the program is straight-line): with eps = 0 the active rows of J must be linearly
+ * independent. Two or more points on one rigid body (toe and heel of one foot: 6 rows of rank 5) are not, and need
+ * eps > 0; the equations above then hold with that eps.
+ * FP64 only. The programs are specialised for the contact set and compiled at run time when first used (GRBDA_JIT=0:
+ * GRBDA_ERR_NOT_COMPILED). One hand-written kernel packs [tau; s; eps] (contact dynamics) or [s; e; eps] (impulse) per
+ * state into the per-stream scratch buffer of the VJP entry points on `stream`, then the program runs on `stream`; that
+ * buffer belongs to the (handle, stream) pair, with the same concurrency caveat. Refused with
+ * GRBDA_ERR_INVALID_ARGUMENT: a model without contact points, batch < 0, a NULL pointer other than `active`, eps < 0
+ * or not finite, e outside [0, 1]; GRBDA_ERR_NO_DEVICE for a host-only handle. batch = 0 returns GRBDA_OK without
+ * launching anything. */
+grbda_status grbda_cuda_contact_forward_dynamics_f64(const grbda_model *m, const double *q, const double *yd,
+                                                     const double *tau, const uint8_t *active, double damping,
+                                                     double *ydd, double *lambda, int64_t batch, void *stream);
+grbda_status grbda_cuda_contact_impulse_f64(const grbda_model *m, const double *q, const double *yd,
+                                            const uint8_t *active, double restitution, double damping, double *yd_plus,
+                                            double *impulse, int64_t batch, void *stream);
 
 /* Derivatives of the dynamics (SURVEY 8 f4). The reference has no closed-form derivative algorithm: it takes
  * CasADi's jacobian() of its symbolic model with respect to a tangent-space perturbation dq of the positions, the
